@@ -1,6 +1,7 @@
 """bench.py -- leapfrog grad-evals/s (and SMC iters/s) of the SMC-NUTS particle hot path on B200.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload arma|PRMwCD|gauss]
+                    [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P \
            bench.py --gpus N --steps K --warmup W
 
@@ -22,6 +23,15 @@ difference of the estimates.
            bounded sample of the SAME particle state.
 `--impl reference`: the oracle port of the whole SMC iteration (the reference is pure Python + BridgeStan, which is
            not installable offline and cannot travel) on the host cores, bounded particle count, same metric.
+`--dump-outputs DIR`: after the timed steps, what the last timed step returned to its caller is written as DIR/<name>.npy
+           (rank 0's shard when sharded): the SMC iteration's particles, log-weights and estimates (`smc_*`) and the
+           last NUTSProposal.rvs call's results (`e2e_*`; `micro_*` for the micro workload).  As in the reference's
+           bookkeeping, smc_x / smc_logw are the particle set AFTER the step's move and reweighting, while
+           smc_mean_estimate, smc_variance_estimate, smc_ess and smc_log_likelihood describe the set the step started
+           from.  Every array is float64, counters (leapfrogs, resampled) and `sample_rows` included.  All inputs derive
+           from fixed seeds, so two builds run with the same arguments can be compared array for array.  At most 64 MB
+           in all: when the per-particle arrays are larger, the same seeded sample of rows is taken from each and its
+           indices are `sample_rows.npy`.
 """
 import argparse
 import json
@@ -135,6 +145,40 @@ def workload_name(workload, model, n_global, lk, temp, eps, resampling):
             f"BASELINE.json configs[{cfg}]")
 
 
+DUMP_BYTES = 63_000_000    # array data of --dump-outputs: under 64 MB with the .npy headers
+
+
+def _host(v, rows=None):
+    """float64 NumPy copy of a NumPy array, a host or device tensor or a scalar; `rows` selects along the first axis."""
+    if hasattr(v, "index_select"):
+        import torch
+        if rows is not None:
+            v = v.index_select(0, torch.as_tensor(rows, device=v.device))
+        v = v.cpu().numpy()
+    elif rows is not None:
+        v = np.asarray(v)[rows]
+    return np.asarray(v, dtype=np.float64)
+
+
+def dump_outputs(out_dir, per_particle, scalars):
+    """--dump-outputs: `scalars` (estimates, counters) are written whole; the `per_particle` arrays (one row per particle)
+    keep every row if everything fits in DUMP_BYTES, otherwise the same fixed seeded sample of rows each."""
+    out = Path(out_dir)
+    out.mkdir(parents=True, exist_ok=True)
+    small = {k: _host(v) for k, v in scalars.items()}
+    n = len(next(iter(per_particle.values())))
+    row_bytes = 8 * sum(int(np.prod(v.shape[1:])) for v in per_particle.values())
+    rows = min(n, (DUMP_BYTES - sum(a.nbytes for a in small.values())) // (row_bytes + 8))
+    idx = None
+    if rows < n:
+        idx = np.sort(np.random.default_rng(0).choice(n, rows, replace=False))
+        small["sample_rows"] = idx.astype(np.float64)
+    for k, v in per_particle.items():
+        np.save(out / f"{k}.npy", _host(v, idx))
+    for k, a in small.items():
+        np.save(out / f"{k}.npy", a)
+
+
 def run_reference(args):
     """Reference arm: the oracle port of the SMC iteration on the host cores (all threads)."""
     rank = int(os.environ.get("RANK", "0"))
@@ -167,6 +211,12 @@ def run_reference(args):
     for k in range(args.warmup, args.warmup + args.steps):
         smc.step(k)
     dt = time.perf_counter() - t0
+    if args.dump_outputs:
+        k = args.warmup + args.steps - 1
+        dump_outputs(args.dump_outputs, {"smc_x": smc.x, "smc_logw": smc.logw},
+                     {"smc_mean_estimate": smc.mean_estimate[k], "smc_variance_estimate": smc.variance_estimate[k],
+                      "smc_ess": smc.ess[k], "smc_log_likelihood": smc.log_likelihood[k], "smc_phi": smc.phi[k],
+                      "smc_leapfrogs": smc.n_leapfrog[k], "smc_resampled": smc.resampled[k]})
     lf = int(smc.n_leapfrog[args.warmup:].sum())
     val = lf / dt
     n_full = 1 << (args.log2n or log2n)
@@ -267,6 +317,8 @@ def run_micro(args):
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
     dt, per = t[0].item(), t[1:].cpu().numpy()
     clk = clocks.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {"micro_resampled_x": xs}, {"micro_log_z": stats[0], "micro_ess": stats[1]})
     peaks = json.loads((ROOT / "MEASURED_PEAKS.json").read_text()) if (ROOT / "MEASURED_PEAKS.json").exists() else {}
     hbm = float(peaks.get("hbm_gbs", 6650.0))
     if rank == 0:
@@ -311,6 +363,8 @@ def main():
     ap.add_argument("--resampling", default="multinomial", choices=["multinomial", "systematic"])
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-peer-push", action="store_true", help="micro: migrate with NCCL all-to-all-v instead of the fused peer stores")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step computed as DIR/<name>.npy (at most 64 MB in all)")
     args = ap.parse_args()
     if args.workload == "micro":
         return run_micro(args)
@@ -455,6 +509,14 @@ def main():
         dist.all_reduce(le, op=dist.ReduceOp.SUM)
     e2e_val = le.item() / te.item()
     clk = clocks.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        k, s = W + K - 1, smc.samples
+        dump_outputs(args.dump_outputs,
+                     {"smc_x": s.x, "smc_logw": s.logw, "e2e_x_new": xn, "e2e_r_new": rn,
+                      "e2e_n_leapfrog": fk.last["n_leapfrog"]},
+                     {"smc_mean_estimate": smc._mean_dev[k], "smc_variance_estimate": smc._var_dev[k],
+                      "smc_ess": smc.ess[k], "smc_log_likelihood": smc.log_likelihood[k], "smc_phi": smc.phi[k],
+                      "smc_leapfrogs": smc._lf[k], "smc_resampled": smc.resampled[k]})
 
     # ---------------------------------------------------------------- extra key at N > 1: the same iteration, weak scaling
     # (the workload's particle count PER GPU); `value` above stays the strong-scaling number of the stated configuration

@@ -14,7 +14,7 @@ from oracle import smc_oracle as O
 
 ROOT = Path(__file__).resolve().parents[1]
 STAN = ROOT / "tests" / "stan"
-REF_MODELS = Path("/root/reference/stan_models")
+REF_STAN = ROOT / "tests" / "golden" / "reference_stan"
 DATA = ROOT / "smc-nuts_b200" / "smcnuts" / "data"
 
 pytestmark = pytest.mark.skipif(not BT.available(), reason="bridgestan is not installed (offline image)")
@@ -31,8 +31,8 @@ def _data(name):
 
 def _programs(name):
     out = [STAN / {"arma": "arma_series.stan", "PRMwCD": "prm_kernel.stan"}[name]]
-    if (REF_MODELS / name / f"{name}.stan").exists():
-        out.append(REF_MODELS / name / f"{name}.stan")       # the reference's own text, where the checkout is present
+    if (REF_STAN / f"{name}.stan").exists():
+        out.append(REF_STAN / f"{name}.stan")       # the original project's own text, where it is stored
     return out
 
 
