@@ -246,8 +246,9 @@ int smcb_gaussL_gram(const double* r_new, const double* x_new, long long N, int 
  * scratch: 6*D*D doubles. */
 int smcb_gaussL_factor(const double* gram, long long N_total, int D, double ridge, double* G, double* out_logdet,
                        double* scratch, void* stream);
-/* out_i = -0.5*(D log 2pi + logdet + |G (X_i - mean)|^2).  scratch (nullable): 2*D*(D+8) doubles; when given and
- * D <= 104 the GEMM runs on the FP64 tensor cores (mma.m8n8k4). */
+/* out_i = -0.5*(D log 2pi + logdet + |G (X_i - mean)|^2).  scratch (nullable): smcb_gaussL_logpdf_scratch_bytes(D)
+ * bytes; when given and D <= 104 the GEMM runs on the FP64 tensor cores (mma.m8n8k4). */
+long long smcb_gaussL_logpdf_scratch_bytes(int D);
 int smcb_gaussL_logpdf(const double* r_new, const double* x_new, long long N, int D, const double* mean,
                        const double* G, const double* logdet, double* out, double* scratch, void* stream);
 

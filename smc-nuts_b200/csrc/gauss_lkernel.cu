@@ -510,14 +510,24 @@ int smcb_gaussL_factor(const double* gram, long long N_total, int D, double ridg
     return check_launch("gaussL_factor_kernel");
 }
 
+// FP64 tensor-core logpdf (D <= 104): NT8 n-tiles of 8 rows of G, KK k-steps of 4 columns; the packed fragments of G'
+// take NT8 * KK * 32 doubles of the caller's scratch
+static int gaussL_nt8(int D) { return D <= 8 ? 1 : D <= 16 ? 2 : D <= 32 ? 4 : D <= 64 ? 8 : 13; }
+static int gaussL_kk(int D) { return (2 * D + 3) / 4; }
+
+long long smcb_gaussL_logpdf_scratch_bytes(int D) {
+    if (D < 1 || D > 104) return 0;   // scalar path: no scratch
+    return (long long)sizeof(double) * gaussL_nt8(D) * gaussL_kk(D) * 32;
+}
+
 int smcb_gaussL_logpdf(const double* r_new, const double* x_new, long long N, int D, const double* mean,
                        const double* G, const double* logdet, double* out, double* scratch, void* stream) {
     SMCB_REQUIRE(r_new && x_new && mean && G && logdet && out && N >= 0 && D >= 1 && D <= kGDmax, "bad argument (D <= 128)");
     if (N == 0) return 0;
     if (D <= 104 && scratch) {   // FP64 tensor-core path; scratch holds the packed fragments of G'
         cudaStream_t st = (cudaStream_t)stream;
-        const int NT8 = D <= 8 ? 1 : D <= 16 ? 2 : D <= 32 ? 4 : D <= 64 ? 8 : 13;
-        const int KK = (2 * D + 3) / 4;
+        const int NT8 = gaussL_nt8(D);
+        const int KK = gaussL_kk(D);
         const int nfrag = NT8 * KK * 32;
         gaussL_pack_G_kernel<<<(nfrag + 255) / 256, 256, 0, st>>>(G, D, NT8, KK, scratch);
         if (check_launch("gaussL_pack_G_kernel")) return -1;

@@ -58,12 +58,18 @@ __device__ __forceinline__ void tile_half_sqnorm(const double* __restrict__ r, l
 // Cooperative variant for D = 2*LPR (LPR = lanes per row, a power of two): LPR adjacent lanes read one row as
 // 16-byte chunks, so every warp-level load covers 32/LPR whole rows = 512 contiguous bytes; the squares are folded
 // with log2(LPR) shuffles.  ROWS_PER_ITER rows per group are in flight to keep enough bytes outstanding.
+// The groups of one warp can run different trip counts of their row loops, so a shuffle names only its own group's
+// lanes (every xor offset is < LPR: the exchange never leaves the group).
+template <int LPR>
+__device__ __forceinline__ unsigned group_mask() {
+    return LPR == 32 ? 0xffffffffu : ((1u << (LPR & 31)) - 1u) << ((threadIdx.x & 31) & ~(LPR - 1));
+}
 template <int LPR>
 __device__ __forceinline__ double group_half_sqnorm(const double* __restrict__ rowp, int sub) {
     const double2 v = *reinterpret_cast<const double2*>(rowp + 2 * sub);
     double s = v.x * v.x + v.y * v.y;
 #pragma unroll
-    for (int o = LPR / 2; o > 0; o >>= 1) s += __shfl_xor_sync(0xffffffffu, s, o);
+    for (int o = LPR / 2; o > 0; o >>= 1) s += __shfl_xor_sync(group_mask<LPR>(), s, o);
     return 0.5 * s;
 }
 
@@ -93,8 +99,8 @@ __global__ void __launch_bounds__(256) reweight_forward_coop_kernel(const double
         for (int o = LPR / 2; o > 0; o >>= 1)
 #pragma unroll
             for (int u = 0; u < U; ++u) {
-                k0[u] += __shfl_xor_sync(0xffffffffu, k0[u], o);
-                k1[u] += __shfl_xor_sync(0xffffffffu, k1[u], o);
+                k0[u] += __shfl_xor_sync(group_mask<LPR>(), k0[u], o);
+                k1[u] += __shfl_xor_sync(group_mask<LPR>(), k1[u], o);
             }
         if (sub < U) {  // lane `sub` of the group finishes row i0 + sub: coalesced 8-byte scalars
             double kk0 = k0[0], kk1 = k1[0];

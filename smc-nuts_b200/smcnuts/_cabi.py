@@ -77,6 +77,7 @@ _SIGS = {
     "smcb_gaussL_gram": [_vp, _vp, _ll, _i, _vp, _vp, _vp],
     "smcb_gaussL_factor": [_vp, _ll, _i, _d, _vp, _vp, _vp, _vp],
     "smcb_gaussL_logpdf": [_vp, _vp, _ll, _i, _vp, _vp, _vp, _vp, _vp, _vp],
+    "smcb_gaussL_logpdf_scratch_bytes": [_i],
     "smcb_sum_int32": [_vp, _ll, _vp, _vp, _vp],
     "smcb_sum_f64": [_vp, _ll, _vp, _vp, _vp],
     "smcb_constrain_rows": [_vp, _ll, _i, _vp, _vp, _vp],
@@ -94,7 +95,8 @@ _SIGS = {
     "smcb_scan_workspace_bytes": [_ll],
 }
 _RESTYPES = {"smcb_last_error": ctypes.c_char_p, "smcb_launch_count": _ll, "smcb_reduce_workspace_bytes": _ll,
-             "smcb_scan_workspace_bytes": _ll, "smcb_bisect_state_bytes": _ll, "smcb_resample_workspace_bytes": _ll}
+             "smcb_scan_workspace_bytes": _ll, "smcb_bisect_state_bytes": _ll, "smcb_resample_workspace_bytes": _ll,
+             "smcb_gaussL_logpdf_scratch_bytes": _ll}
 
 _LIB = None
 

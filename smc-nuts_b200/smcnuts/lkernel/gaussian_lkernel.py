@@ -37,7 +37,8 @@ class GaussianApproxLKernel:
                    dev.ptr(scratch), st)
         self.last_status = logdet
         out = dev.empty(n)
-        frag = dev.empty(2 * D * (D + 8) + 4096)
+        nfrag = _cabi.lib().smcb_gaussL_logpdf_scratch_bytes(D) // 8
+        frag = dev.empty(nfrag) if nfrag else None   # None: D > 104 takes the scalar kernel, which needs no scratch
         _cabi.call("smcb_gaussL_logpdf", dev.ptr(r), dev.ptr(x), n, D, dev.ptr(mean), dev.ptr(G), dev.ptr(logdet),
                    dev.ptr(out), dev.ptr(frag), st)
         return dev.like_input(out, x_new)

@@ -140,11 +140,12 @@ def gauss_model(dim=100, rho=0.9, precision=None):
     """Synthetic correlated Gaussian (BASELINE.json config 4): Sigma_ij = rho^|i-j|, dense precision."""
     if precision is None:
         idx = np.arange(dim)
-        P = np.linalg.inv(rho ** np.abs(idx[:, None] - idx[None, :]))
-        precision = 0.5 * (P + P.T)
-    precision = np.asarray(precision, dtype=np.float64)
-    dim = precision.shape[0]
-    return DeviceModel("gauss", precision.ravel(), dim, constrained=False)
+        precision = np.linalg.inv(rho ** np.abs(idx[:, None] - idx[None, :]))
+    P = np.asarray(precision, dtype=np.float64)
+    # the kernels read P as given: the plain one forms -P x, the tensor-core one -P'x; with P symmetric both are the
+    # gradient of B = -x'Px/2 (and this is the matrix oracle.models.GaussTarget uses)
+    P = 0.5 * (P + P.T)
+    return DeviceModel("gauss", P.ravel(), P.shape[0], constrained=False)
 
 
 def make_model(name, **kw):
