@@ -57,6 +57,12 @@ int smcb_model_create_plugin(const char* so_path, const double* host_data, long 
 int smcb_model_set_scale(void* handle, const double* host_scale);
 int smcb_model_destroy(void* handle);
 int smcb_model_dim(void* handle);
+/* Constrained output of a plug-in model (replaces StanModel.constrain, bridgestan.py:93-120: param_constrain per particle,
+ * param_num() values per row).  smcb_model_constrained_dim returns the row width CDIM (a simplex[K] has K - 1 unconstrained
+ * coordinates but K values; -1 with an error for a built-in model, whose transform is fused into the moment kernels).
+ * smcb_model_constrain writes out[N, CDIM] row-major (device) from the unconstrained rows x[N, dim] (device), on stream. */
+int smcb_model_constrained_dim(void* handle);
+int smcb_model_constrain(void* handle, const double* x, long long N, double* out, void* stream);
 /* Host-only test hook (no GPU work): the tensor-core fragment packing of the PRMwCD NUTS kernel (csrc/models.cuh,
  * PrmModelG) applied to a scalar blob [16 header doubles][n_obs rows of 12]; host_out gets 32 + tiles*288 doubles. */
 int smcb_debug_pack_prm(const double* host_scalar_blob, int n_obs, int tiles, double* host_out, long long n_out);
@@ -210,12 +216,8 @@ int smcb_peer_free(void* ptr);
 /* out[j, :] = x[idx[j], :]  (samples.py:140) */
 int smcb_gather_rows(const double* x, const int64_t* idx, long long M, int D, double* out, void* stream);
 
-/* out[i][d] = Stan's constraining transform of x[i][d] (bridgestan.py:93-120 calls param_constrain per particle).
- * table (device, 3*D doubles): per coordinate kind (0 identity, 1 lower: lo + exp u, 2 upper: hi - exp u, 3 both:
- * lo + (hi - lo) inv_logit u), lo, hi.  Used for generated models; the built-in ones fuse exp-on-last into the moments. */
 /* out[i][d] = x[i][d] * scale[d] (inverse = 0) or x[i][d] / scale[d] (inverse = 1); scale is a device array of D doubles */
 int smcb_scale_rows(const double* x, long long N, int D, const double* scale, int inverse, double* out, void* stream);
-int smcb_constrain_rows(const double* x, long long N, int D, const double* table, double* out, void* stream);
 
 /* ---- estimators (estimate.py:79-95 with constrain fused, bridgestan.py:93-120) */
 /* out[d] = sum_i wn_i * (c(x_i)_d - center_d)^power ; center may be NULL (0), power in {1, 2} */

@@ -44,7 +44,9 @@ inline int check_launch(const char* where) {
         if (!(cond)) return ::smcb::fail(__func__, msg); \
     } while (0)
 
-// Entry points of a generated model plug-in (nuts_plugin.cuh), resolved by smcb_model_create_plugin
+// Entry points of a generated model plug-in (nuts_plugin.cuh), resolved by smcb_model_create_plugin; a plug-in built
+// against another version of this table is refused
+#define SMCB_PLUGIN_ABI 2
 struct NutsArgs;
 struct PluginVT {
     void* dl;
@@ -55,6 +57,8 @@ struct PluginVT {
     long long (*nuts_workspace_bytes)(const ModelDesc*, long long, int);
     int (*nuts_transition)(const ModelDesc*, const NutsArgs*, long long, void*);
     int (*logp_grad)(const ModelDesc*, const double*, long long, double, double*, double*, double*, void*);
+    int (*constrained_dim)(void);
+    int (*constrain)(const ModelDesc*, const double*, long long, double*, void*);
 };
 
 struct Model {

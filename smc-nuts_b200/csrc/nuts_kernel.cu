@@ -118,9 +118,11 @@ int smcb_model_create_plugin(const char* so_path, const double* host_data, long 
     vt->nuts_workspace_bytes = (long long (*)(const ModelDesc*, long long, int))sym("smcb_plugin_nuts_workspace_bytes");
     vt->nuts_transition = (int (*)(const ModelDesc*, const NutsArgs*, long long, void*))sym("smcb_plugin_nuts_transition");
     vt->logp_grad = (int (*)(const ModelDesc*, const double*, long long, double, double*, double*, double*, void*))sym("smcb_plugin_logp_grad");
+    vt->constrained_dim = (int (*)(void))sym("smcb_plugin_constrained_dim");
+    vt->constrain = (int (*)(const ModelDesc*, const double*, long long, double*, void*))sym("smcb_plugin_constrain");
     auto bail = [&](const char* what) { dlclose(dl); delete vt; return fail("smcb_model_create_plugin", what); };
     if (!ok) return bail("not a model plug-in: an smcb_plugin_* entry point is missing (csrc/nuts_plugin.cuh)");
-    if (vt->abi() != 1) return bail("plug-in ABI version mismatch: rebuild it against this library's csrc/");
+    if (vt->abi() != SMCB_PLUGIN_ABI) return bail("plug-in ABI version mismatch: rebuild it against this library's csrc/");
     if (vt->ndata() != n) return bail("data blob length differs from the one the plug-in was generated for");
     ModelDesc d{};
     d.kind = kPlugin;
@@ -171,6 +173,21 @@ int smcb_model_destroy(void* handle) {
 }
 
 int smcb_model_dim(void* handle) { return handle ? ((Model*)handle)->desc.dim : -1; }
+
+int smcb_model_constrained_dim(void* handle) {
+    SMCB_REQUIRE(handle && ((Model*)handle)->vt, "bad argument: built-in models constrain inside the moment kernels");
+    return ((Model*)handle)->vt->constrained_dim();
+}
+
+int smcb_model_constrain(void* handle, const double* x, long long N, double* out, void* stream) {
+    SMCB_REQUIRE(handle && ((Model*)handle)->vt, "bad argument: built-in models constrain inside the moment kernels");
+    SMCB_REQUIRE(x && out && N >= 0, "bad argument");
+    if (N == 0) return 0;
+    const Model* m = (const Model*)handle;
+    if (m->vt->constrain(&m->desc, x, N, out, stream)) return fail("smcb_model_constrain (plug-in)", m->vt->last_error());
+    g_launches.fetch_add(1, std::memory_order_relaxed);
+    return 0;
+}
 
 int smcb_debug_pack_prm(const double* host_scalar_blob, int n_obs, int tiles, double* host_out, long long n_out) {
     SMCB_REQUIRE(host_scalar_blob && host_out && n_obs > 0 && tiles > 0 && n_obs <= 8 * tiles, "bad argument");

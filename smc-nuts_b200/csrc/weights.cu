@@ -716,22 +716,6 @@ __global__ void __launch_bounds__(kRedThreads) sum_kernel(const T* __restrict__ 
     }
 }
 
-// Stan's constraining transforms, coordinate by coordinate (generated models: smcnuts/model/stan_codegen.py).
-// table[3 * D]: kind (0 identity, 1 lower, 2 upper, 3 lower and upper), lo, hi per coordinate.
-__global__ void constrain_rows_kernel(const double* __restrict__ x, long long n_elem, int D, const double* __restrict__ table,
-                                      double* __restrict__ out) {
-    for (long long e = blockIdx.x * (long long)blockDim.x + threadIdx.x; e < n_elem; e += (long long)gridDim.x * blockDim.x) {
-        const int col = (int)(e % D);
-        const int kind = (int)table[3 * col];
-        const double lo = table[3 * col + 1], hi = table[3 * col + 2], u = x[e];
-        double v = u;
-        if (kind == 1) v = lo + exp(u);
-        else if (kind == 2) v = hi - exp(u);
-        else if (kind == 3) v = lo + (hi - lo) * (u >= 0.0 ? 1.0 / (1.0 + exp(-u)) : exp(u) / (1.0 + exp(u)));
-        out[e] = v;
-    }
-}
-
 // out[i][d] = x[i][d] * scale[d] (inverse = 0) or x[i][d] / scale[d] (inverse = 1): the change of variables of the
 // diagonal-metric NUTS path (ScaledModel, models.cuh) at the kernel's boundaries
 __global__ void scale_rows_kernel(const double* __restrict__ x, long long n_elem, int D, const double* __restrict__ scale,
@@ -1044,13 +1028,6 @@ int smcb_scale_rows(const double* x, long long N, int D, const double* scale, in
     if (N == 0) return 0;
     scale_rows_kernel<<<stride_grid(N * D, 256, 8), 256, 0, (cudaStream_t)stream>>>(x, N * D, D, scale, inverse, out);
     return check_launch("scale_rows_kernel");
-}
-
-int smcb_constrain_rows(const double* x, long long N, int D, const double* table, double* out, void* stream) {
-    SMCB_REQUIRE(x && table && out && N >= 0 && D >= 1, "bad argument");
-    if (N == 0) return 0;
-    constrain_rows_kernel<<<stride_grid(N * D, 256, 8), 256, 0, (cudaStream_t)stream>>>(x, N * D, D, table, out);
-    return check_launch("constrain_rows_kernel");
 }
 
 int smcb_weighted_moments12(const double* x, const double* wn, long long N, int D, int constrain, const double* center,

@@ -12,7 +12,7 @@ HEADER = _PKG.parents[1] / "include" / "smcnuts_b200.h"
 MODEL_KINDS = {"arma": 0, "PRMwCD": 1, "gauss": 2}
 STREAM_NUTS, STREAM_MOMENTUM, STREAM_ACCREJ, STREAM_RESAMPLE, STREAM_INIT, STREAM_ESTIMATE = range(6)
 CONSTRAIN_NONE, CONSTRAIN_EXP_LAST = 0, 1
-CONSTRAIN_TABLE = 2   # host side only: constrain with smcb_constrain_rows first, then unconstrained moments
+CONSTRAIN_MODEL = 2   # host side only: constrain through the model (smcb_model_constrain) first, then unconstrained moments
 
 _vp, _ll, _i, _d = ctypes.c_void_p, ctypes.c_longlong, ctypes.c_int, ctypes.c_double
 _u64, _u32 = ctypes.c_uint64, ctypes.c_uint32
@@ -24,6 +24,8 @@ _SIGS = {
     "smcb_model_set_scale": [_vp, _vp],
     "smcb_model_destroy": [_vp],
     "smcb_model_dim": [_vp],
+    "smcb_model_constrained_dim": [_vp],
+    "smcb_model_constrain": [_vp, _vp, _ll, _vp, _vp],
     "smcb_debug_pack_prm": [_vp, _i, _i, _vp, _ll],
     "smcb_logp_grad": [_vp, _vp, _ll, _d, _vp, _vp, _vp, _vp],
     "smcb_combine_logp": [_vp, _vp, _d, _ll, _vp, _vp],
@@ -80,7 +82,6 @@ _SIGS = {
     "smcb_gaussL_logpdf_scratch_bytes": [_i],
     "smcb_sum_int32": [_vp, _ll, _vp, _vp, _vp],
     "smcb_sum_f64": [_vp, _ll, _vp, _vp, _vp],
-    "smcb_constrain_rows": [_vp, _ll, _i, _vp, _vp, _vp],
     "smcb_scale_rows": [_vp, _ll, _i, _vp, _i, _vp, _vp],
     "smcb_fast_exp": [_vp, _ll, _vp, _vp],
     "smcb_fast_log": [_vp, _ll, _vp, _vp],

@@ -20,7 +20,7 @@ class Estimate:
     def return_estimate(self, x, wn, center=None):
         """center (device tensor [D], optional): a point near the mean, e.g. the previous iteration's estimate -- the two
         moments then come from ONE pass over the particles and one collective (same estimates to rounding)."""
-        if center is not None and self._constrain != _cabi.CONSTRAIN_TABLE and 2 * x.shape[1] <= 256 and not dev.is_host(x):
+        if center is not None and self._constrain != _cabi.CONSTRAIN_MODEL and 2 * x.shape[1] <= 256 and not dev.is_host(x):
             return self._estimate_one_pass(x, wn, self._constrain, center)
         return self._estimate(x, wn, self._constrain)
 
@@ -39,9 +39,9 @@ class Estimate:
 
     def _estimate(self, x, wn, constrain=_cabi.CONSTRAIN_NONE):
         xd, wd = dev.to_device(x), dev.to_device(wn)
-        N, D = xd.shape
-        if constrain == _cabi.CONSTRAIN_TABLE:     # generated models: Stan's transforms coordinate by coordinate
+        if constrain == _cabi.CONSTRAIN_MODEL:     # generated models: [N, dim] -> [N, constrained_dim] through the plug-in
             xd, constrain = self.target.constrain(xd), _cabi.CONSTRAIN_NONE
+        N, D = xd.shape
         mean, var = dev.empty(D), dev.empty(D)
         ws, st = dev.reduce_ws(), dev.stream_ptr()
         _cabi.call("smcb_weighted_moment", dev.ptr(xd), dev.ptr(wd), N, D, constrain, 0, 1, dev.ptr(mean),

@@ -17,7 +17,7 @@ class EstimateFromTempered(Estimate):
         self.resampler = Resampler(N, self.seed, self.shard, stream=_cabi.STREAM_ESTIMATE, scheme=resampling)
 
     def estimate_from_tempered(self, x_saved, logw_saved, phi):
-        D = self.target.dim
+        D = getattr(self.target, "constrained_dim", self.target.dim)     # estimates are on the constrained scale
         host = dev.is_host(x_saved)
         mean_e, var_e = np.zeros([self.K + 1, D]), np.zeros([self.K + 1, D])
         for k in range(self.K + 1):

@@ -24,7 +24,6 @@ PKG = Path(__file__).resolve().parents[1]
 CSRC = PKG.parent / "csrc"
 GEN_DIR = PKG / "_lib" / "gen"
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17", "-Xcompiler", "-fPIC", "-shared"]
-_KIND_CODE = {"none": 0.0, "lower": 1.0, "upper": 2.0, "both": 3.0}
 
 
 def _csrc_digest():
@@ -85,35 +84,34 @@ class GeneratedModel(DeviceModel):
         _cabi.call("smcb_model_create_plugin", str(self.so_path).encode(), blob.ctypes.data if blob.size else None, blob.size,
                    ctypes.byref(h))
         self._h = h
+        # constrained names in BridgeStan's form (a simplex[K] theta gives theta.1 ... theta.K) and the dim unconstrained ones
         self.param_names = list(self.source.param_names)
+        self.param_unc_names = list(self.source.param_unc_names)
         # BridgeStan's constrain() appends transformed parameters and generated quantities (bridgestan.py:24,93-120 of the
         # reference: param_num(include_tp=True, include_gq=True)); here they enter the density (transformed parameters) or
         # are skipped (generated quantities) but are NOT appended: estimates cover the declared parameters only
-        self.constrained_dim = self.dim
+        self.constrained_dim = _cabi.lib().smcb_model_constrained_dim(self._h)
+        assert self.constrained_dim == self.source.cdim, (self.constrained_dim, self.source.cdim)
         kinds = [t[0] for t in self.source.transforms]
         if all(k == "none" for k in kinds):
             self.constrain_kind = _cabi.CONSTRAIN_NONE
         elif kinds[-1] == "lower" and self.source.transforms[-1][1] == 0.0 and all(k == "none" for k in kinds[:-1]):
             self.constrain_kind = _cabi.CONSTRAIN_EXP_LAST       # the fused exp-on-last moments of the built-in models
         else:
-            self.constrain_kind = _cabi.CONSTRAIN_TABLE
-        self._table_host = np.array([[_KIND_CODE[k], lo if lo is not None else 0.0, hi if hi is not None else 0.0]
-                                     for k, lo, hi in self.source.transforms], dtype=np.float64)
-        self._table_dev = None
+            self.constrain_kind = _cabi.CONSTRAIN_MODEL
 
     @classmethod
     def from_files(cls, model_path, data_path=None, name=None):
         return cls(Path(model_path).read_text(), stan_codegen.load_data(data_path), name or Path(model_path).stem)
 
     def constrain(self, x, include_tparams=True, include_gqs=True):
-        """Stan's constraining transforms of the declared parameters (bridgestan.py:93-120), one kernel for the whole
-        particle array; `include_tparams` / `include_gqs` are accepted and ignored (see __init__)."""
-        xd = dev.to_device(x).reshape(-1, self.dim)
-        if self._table_dev is None:
-            self._table_dev = dev.to_device(self._table_host.ravel())
-        out = dev.empty(*xd.shape)
-        _cabi.call("smcb_constrain_rows", dev.ptr(xd), xd.shape[0], self.dim, dev.ptr(self._table_dev), dev.ptr(out),
-                   dev.stream_ptr())
+        """Stan's constraining transforms of the declared parameters (bridgestan.py:93-120): [..., dim] -> [...,
+        constrained_dim], one kernel of the model's plug-in for the whole particle array; `include_tparams` /
+        `include_gqs` are accepted and ignored (see __init__)."""
+        xd = dev.to_device(x).reshape(-1, self.dim).contiguous()
+        out = dev.empty(xd.shape[0], self.constrained_dim)
+        _cabi.call("smcb_model_constrain", self._h, dev.ptr(xd), xd.shape[0], dev.ptr(out), dev.stream_ptr())
+        shape = tuple(np.shape(x)[:-1]) + (self.constrained_dim,)
         if dev.is_host(x):
-            return dev.to_numpy(out).reshape(np.shape(x))
-        return out.reshape(x.shape)
+            return dev.to_numpy(out).reshape(shape)
+        return out.reshape(shape)

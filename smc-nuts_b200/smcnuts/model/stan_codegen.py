@@ -9,7 +9,13 @@ compiles with plain g++ -- that is how the `not gpu` tests check it against the 
 
 What is generated
   * parameters on the unconstrained scale, Stan's transforms and log-Jacobians (lower -> lo + exp(u), upper,
-    lower+upper -> scaled inverse logit), declaration order = BridgeStan's unconstrained order;
+    lower+upper -> scaled inverse logit; simplex, ordered and positive_ordered vectors through csrc/stan_transforms.cuh),
+    declaration order = BridgeStan's unconstrained order.  The body sees one leaf per CONSTRAINED value (c[0 .. CDIM)) and
+    accumulates its gradient over them; after the body one pullback per vector parameter maps it to the unconstrained
+    coordinates and adds the gradient of its log-Jacobian (O(K) per vector, all Jacobians in A).  simplex is Stan's
+    stick-breaking transform of releases up to 2.35 (what BridgeStan builds against those compute); later releases
+    may use another simplex transform, which tests/test_bridgestan_pin.py would show.  The struct's static constrain(x, out)
+    writes the CDIM constrained values with the same transform functions (smcb_model_constrain);
   * the split  logp(x, phi) = A(x) + phi * B(x): the data variable named `phi` is the tempering parameter
     (bridgestan.py:122-146 rewrites it in the data JSON); `target += phi * e` accumulates into B, everything else into A;
     all normalising constants of `target +=` statements are kept, `~` statements drop parameter-free terms (Stan's
@@ -23,19 +29,24 @@ Supported subset (anything else raises StanSubsetError with the offending line):
   blocks functions (functions returning real, inlined at the call: no recursion, one return at the end) / data /
   transformed data / parameters / transformed parameters / model (generated quantities is skipped: it never enters the
   log density);  int, real, vector, row_vector, matrix (data and
-  locals), array[..] (and the pre-2.33 `real y[N]` form);  lower/upper bounds on real parameters;  local declarations
+  locals), array[..] (and the pre-2.33 `real y[N]` form);  lower/upper bounds on real parameters;  simplex[K], ordered[K],
+  positive_ordered[K] (and arrays of them) as parameters, as data (validated at generation time: rows >= 0 summing to 1
+  within 1e-8, strictly increasing) and as plain vectors in transformed parameters;  local declarations
   with initialisers, =, +=, -=, *=, /=, `target +=`, `~`, for and while loops, print (ignored), reject (the density becomes -inf, which is what the
   reference makes of a Stan exception), if / else (conditions on data, loop variables or
   parameter values; && || !), blocks;
   + - * / ^ .* ./, unary minus, indexing, exp log log1p sqrt fabs abs square inv inv_logit log1p_exp log_sum_exp(a, b)
   pow fmin fmax tanh sin cos lgamma (of data: tabulated at generation time; of parameters: differentiated with a digamma series);
   container-valued expressions: elementwise arithmetic and functions, matrix * vector, row_vector * vector,
-  row_vector * matrix, sum mean dot_product dot_self rep_vector rep_row_vector rep_array,
+  row_vector * matrix, sum mean dot_product dot_self rep_vector rep_row_vector rep_array, log_sum_exp(container) (max
+  shifted; gradient = the softmax weights),
   whole-container assignment -- lowered onto element loops and accumulator locals of the scalar subset (`lower_stmt`);
   normal, std_normal, cauchy, student_t, double_exponential, logistic, lognormal, exponential, gamma, inv_gamma, weibull,
   beta, uniform densities; poisson, poisson_log, bernoulli, bernoulli_logit, binomial, binomial_logit, neg_binomial_2,
   neg_binomial_2_log mass functions --
-  scalar or vectorised over container arguments and container-valued argument expressions.
+  scalar or vectorised over container arguments and container-valued argument expressions;  dirichlet (alpha data or
+  parameters), categorical (an int or int array outcome) and multinomial (an int array) of a vector argument, the integer
+  outcomes being data known at generation time (tabulated into counts).
 """
 import json
 import math
@@ -83,6 +94,7 @@ class _Parser:
         self.t = _tokenize(text)
         self.i = 0
         self.orients = {}       # variable name -> "col" (vector) | "row" (row_vector) | "mat" (matrix): how `*` treats it
+        self.ctypes = {}        # variable name -> "simplex" | "ordered" | "positive_ordered"
 
     def peek(self, k=0):
         return self.t[self.i + k]
@@ -188,8 +200,13 @@ class _Parser:
         self.expect("}")
         return name[1], ("real", params, body, line)
 
-    # ---- declarations: (name, base, shape[list of expr], lower, upper, init)
-    _TYPES = ("int", "real", "vector", "row_vector", "array", "matrix")
+    # ---- declarations: (name, base, shape[list of expr], lower, upper, init);  the constrained vector types are vectors
+    #      whose kind is recorded in `ctypes` (name -> kind): enforced for parameters and data, plain vectors elsewhere
+    _VECTOR_TYPES = ("simplex", "ordered", "positive_ordered")
+    _REFUSED_TYPES = ("unit_vector", "sum_to_zero_vector", "sum_to_zero_matrix", "cholesky_factor_corr",
+                      "cholesky_factor_cov", "cov_matrix", "corr_matrix", "column_stochastic_matrix",
+                      "row_stochastic_matrix")
+    _TYPES = ("int", "real", "vector", "row_vector", "array", "matrix") + _VECTOR_TYPES + _REFUSED_TYPES
 
     def is_decl(self):
         return self.peek()[1] in self._TYPES
@@ -228,6 +245,13 @@ class _Parser:
         if base == "array":
             shape += self.dims()
             base = self.next()[1]
+        if base in self._REFUSED_TYPES:
+            raise StanSubsetError(f"line {line}: type {base!r} is outside the supported subset")
+        ctype = None
+        if base in self._VECTOR_TYPES:
+            if self.peek()[1] == "<":
+                raise StanSubsetError(f"line {line}: bounds on a {base} are outside the supported subset")
+            ctype, base = base, "vector"
         lo, hi = self.bounds()
         orient = None
         if base in ("vector", "row_vector", "matrix"):
@@ -242,6 +266,8 @@ class _Parser:
             raise StanSubsetError(f"line {line}: expected a variable name, found {name[1]!r}")
         if orient:
             self.orients[name[1]] = orient
+        if ctype:
+            self.ctypes[name[1]] = ctype
         shape += self.dims()          # pre-2.33 array syntax: real y[N]
         init = self.expr() if self.accept("=") else None
         self.expect(";")
@@ -563,6 +589,17 @@ _DENSITIES = {
                                               _add(_un("lgamma", _add(k, _const(1.0))), _un("lgamma", _add(_sub(n, k), _const(1.0))))),
                                          _mul(k, eta), _un("neg", _mul(n, _un("log1p_exp", eta)))],
 }
+# densities of a whole vector argument (simplex-valued or counts), lowered by _Gen.vector_density
+_VECTOR_DENSITIES = ("dirichlet", "categorical", "multinomial")
+
+
+def _sum_exprs(terms, line):
+    out = terms[0] if terms else ("num", 0.0, True)
+    for t in terms[1:]:
+        out = ("bin", "+", out, t)
+    return out
+
+
 _UNARY_FUNCS = {"exp": "exp", "log": "log", "log1p": "log1p", "sqrt": "sqrt", "fabs": "fabs", "abs": "fabs", "lgamma": "lgamma",
                 "tanh": "tanh", "sin": "sin", "cos": "cos", "inv_logit": "inv_logit", "log1p_exp": "log1p_exp"}
 
@@ -772,17 +809,19 @@ class _Var:
 class GeneratedSource:
     """Result of `generate`: C++ text of the model struct and what the host side needs to know about it."""
 
-    def __init__(self, struct_name, text, dim, blob, param_names, transforms, digest):
+    def __init__(self, struct_name, text, dim, blob, param_names, transforms, digest, cdim, param_unc_names):
         self.struct_name, self.text, self.dim, self.blob = struct_name, text, dim, blob
         self.param_names, self.transforms, self.digest = param_names, transforms, digest
+        self.cdim, self.param_unc_names = cdim, param_unc_names      # constrained width, unconstrained names
 
 
 class _Gen:
     MAX_DIM = 64
 
-    def __init__(self, blocks, data, struct_name, orients=None):
+    def __init__(self, blocks, data, struct_name, orients=None, ctypes=None):
         self.blocks, self.struct_name = blocks, struct_name
         self.orients = orients or {}
+        self.ctypes = ctypes or {}
         self.lowered = {}       # id(statement) -> its scalar-subset replacement (list of statements) or None
         self.fresh = 0
         self.functions = blocks.get("functions", {})
@@ -809,8 +848,12 @@ class _Gen:
         self.indent = 2
         self.tmp = 0
         self.derived = {}       # (data array, shift) -> blob offset of its tabulated lgamma
-        self.transforms = []    # per unconstrained coordinate: (kind, lo, hi) with kind in none/lower/upper/both
-        self.param_names = []
+        self.transforms = []    # per unconstrained coordinate: (kind, lo, hi) with kind in none/lower/upper/both or the
+        #                         vector type (simplex / ordered / positive_ordered) the coordinate belongs to
+        self.param_names = []   # constrained names, BridgeStan's form (theta.1 ... theta.K)
+        self.param_unc_names = []
+        self.blocks_of = []     # per parameter transform, in declaration order: (kind, lo, hi, unconstrained offset,
+        #                         constrained offset, K) -- K = 1 for a scalar coordinate
 
     # ---- integer expressions (indices, bounds, sizes): folded to Python ints when no loop variable is involved
     def int_expr(self, e):
@@ -1031,7 +1074,8 @@ class _Gen:
             raise StanSubsetError(f"operator {op} between two containers is outside the supported subset")
         if k == "call":
             name, args = e[1], e[2]
-            if name in self._REDUCTIONS or name in self.functions or re.fullmatch(r"\w+_(lpdf|lpmf|log)", name):
+            if (name in self._REDUCTIONS or name in self.functions or re.fullmatch(r"\w+_(lpdf|lpmf|log)", name)
+                    or (name == "log_sum_exp" and len(args) == 1)):
                 return (), None
             if name in self._REPS and len(args) == 2:
                 n, _ = self.int_expr(args[1])
@@ -1111,7 +1155,11 @@ class _Gen:
                 return ("bin", "/", total, ("num", float(n), False)) if name == "mean" else total
             if name in self.functions:
                 return self.lower(self.inline(name, args, pre, cl), [], pre, cl)
+            if name == "log_sum_exp" and len(args) == 1:
+                return self.log_sum_exp(args[0], pre, cl)
             m = re.fullmatch(r"(\w+?)_(lpdf|lpmf|log)", name)
+            if m and m.group(1) in _VECTOR_DENSITIES:
+                return _sum_exprs(self.vector_density(m.group(1), args, pre, cl), cl)
             if m and m.group(1) in _DENSITIES:
                 shapes = [self.shape(a)[0] for a in args]
                 big = [d for d in shapes if d]
@@ -1123,6 +1171,88 @@ class _Gen:
                 return ("call", name, [self.lower(a, [], pre, cl) for a in args], cl)
             return ("call", name, [self.lower(a, ix if self.shape(a)[0] else [], pre, cl) for a in args], cl)
         raise StanSubsetError(f"unsupported expression {e!r}")
+
+    def one_dim(self, e, what, line):
+        dims, _ = self.shape(e)
+        if len(dims) != 1:
+            raise StanSubsetError(f"line {line}: {what} takes a one-dimensional container")
+        return dims[0]
+
+    def log_sum_exp(self, v, pre, line):
+        """log sum_k exp(v_k) = m + log sum_k exp(v_k - m) with m = max_k v_k; its gradient is the softmax weights (the
+        derivatives through m cancel)"""
+        n = self.one_dim(v, "log_sum_exp", line)
+        mx, kv = self.fresh_name("m"), self.fresh_name("k")
+        inner = []
+        elem = self.lower(v, [("var", kv, line)], inner, line)
+        pre.append(("decl", (mx, "real", [], None, None, self.lower(v, [("num", 1.0, True)], pre, line), line), line))
+        pre.append(("for", kv, ("num", 2.0, True), ("num", float(n), True),
+                    [("block", inner + [("assign", ("var", mx, line), "=", ("call", "fmax", [("var", mx, line), elem], line),
+                                         line)], line)], line))
+        total = self.reduce(n, lambda kk, p2: ("call", "exp", [("bin", "-", self.lower(v, [kk], p2, line), ("var", mx, line))],
+                                               line), pre, line)
+        return ("bin", "+", ("var", mx, line), ("call", "log", [total], line))
+
+    def data_ints(self, e, what, line):
+        """values of an integer data expression (a scalar, an array, or an element), known at generation time"""
+        base, idx = (e, []) if e[0] == "var" else (e[1], e[2]) if e[0] == "idx" else (None, None)
+        v = self.vars.get(base[1]) if base is not None and base[0] == "var" else None
+        if v is None or v.kind != "data" or v.base != "int" or self.is_loop_var(base[1]):
+            raise StanSubsetError(f"line {line}: the outcome of {what} must be integer data (an index known when the "
+                                  f"model is generated)")
+        if not v.shape:
+            return [v.value]
+        if len(idx) == len(v.shape):
+            iv, _ = self.flat_index(v, idx, line)
+            if iv is None:
+                raise StanSubsetError(f"line {line}: the outcome of {what} must not depend on a loop variable")
+            return [int(v.value[iv])]
+        if idx:
+            raise StanSubsetError(f"line {line}: the outcome of {what} must be a whole array or one element")
+        return [int(z) for z in v.value]
+
+    def vector_density(self, dist, args, pre, line):
+        """dirichlet_lpdf(theta | alpha), categorical_lpmf(y | theta), multinomial_lpmf(y | theta) as scalar-subset
+        expressions -> the list of its terms; with the integer outcomes tabulated into counts at generation time they
+        all read sum_k c_k log theta_k plus normalising terms."""
+        if len(args) != 2:
+            raise StanSubsetError(f"line {line}: {dist} takes 2 arguments")
+
+        def log_elem(e, k):
+            return ("call", "log", [self.lower(e, [("num", float(k), True)], pre, line)], line)
+
+        def weighted_logs(e, counts):
+            terms = [("bin", "*", ("num", float(c), True), log_elem(e, k + 1)) for k, c in enumerate(counts) if c]
+            return _sum_exprs(terms, line)
+
+        if dist == "dirichlet":
+            theta, alpha = args
+            K = self.one_dim(theta, "dirichlet", line)
+            if self.one_dim(alpha, "dirichlet", line) != K:
+                raise StanSubsetError(f"line {line}: dirichlet arguments have different sizes")
+            a = lambda kk: self.lower(alpha, [kk], pre, line)     # noqa: E731
+            total = self.reduce(K, lambda kk, p2: self.lower(alpha, [kk], p2, line), pre, line)
+            lg = self.reduce(K, lambda kk, p2: ("call", "lgamma", [self.lower(alpha, [kk], p2, line)], line), pre, line)
+            body = []
+            for k in range(1, K + 1):
+                ak = a(("num", float(k), True))
+                if not (ak[0] == "idx" and self.vars.get(ak[1][1]) is not None and self.vars[ak[1][1]].kind == "data"
+                        and self.real(ak).kind == "const" and self.real(ak).val == 1.0):     # (1 - 1) log theta_k: no term
+                    body.append(("bin", "*", ("bin", "-", ak, ("num", 1.0, True)), log_elem(theta, k)))
+            body = _sum_exprs(body, line)
+            return [("call", "lgamma", [total], line), ("neg", lg), body]
+        y, theta = args
+        K = self.one_dim(theta, dist, line)
+        ys = self.data_ints(y, dist, line)
+        if any(not (1 <= z <= K) for z in ys) and dist == "categorical":
+            raise StanSubsetError(f"line {line}: categorical outcomes must lie in 1..{K}")
+        if dist == "categorical":
+            counts = [sum(1 for z in ys if z == k) for k in range(1, K + 1)]
+            return [weighted_logs(theta, counts)]
+        if len(ys) != K or any(z < 0 for z in ys):
+            raise StanSubsetError(f"line {line}: multinomial counts must be {K} non-negative integers")
+        norm = math.lgamma(sum(ys) + 1.0) - math.fsum(math.lgamma(z + 1.0) for z in ys)
+        return [("num", norm, False), weighted_logs(theta, ys)]
 
     def is_plain(self, e):
         """Expressions the scalar machinery takes as they are: scalars without container operations inside, and whole
@@ -1181,6 +1311,8 @@ class _Gen:
                 dist, args = (m.group(1), e[2]) if (m and m.group(1) in _DENSITIES) else (None, None)
             else:
                 tempered, dist, args = False, s[2], [s[1]] + s[3]
+                if dist in _VECTOR_DENSITIES:       # propto: a term that depends on no parameter is dropped when emitted
+                    return pre + [("ptarget", t, line) for t in self.vector_density(dist, args, pre, line)]
 
             def rebuild(a):
                 if kind == "tilde":
@@ -1390,7 +1522,7 @@ class _Gen:
             if not (mm and mm.group(1) in _DENSITIES):
                 return None
             args = list(e[2])
-        elif st[0] == "tilde":
+        elif st[0] == "tilde" and st[2] in _DENSITIES:
             args = [st[1]] + list(st[3])
         else:
             return None
@@ -1822,6 +1954,9 @@ class _Gen:
             elif kind == "target":
                 if emit:
                     self.target_terms(s[1], line, drop_constant_terms=False)
+            elif kind == "ptarget":      # one term of a `~` statement (vector densities): dropped when parameter-free
+                if emit:
+                    self.target_terms(s[1], line, drop_constant_terms=True)
             elif kind == "tilde":
                 if emit:
                     _, lhs, dist, args, _ = s
@@ -1860,13 +1995,17 @@ class _Gen:
                     n *= d
                 if len(flat) != n:
                     raise StanSubsetError(f"data {name!r}: expected {n} values, found {len(flat)}")
+                if name in self.ctypes:
+                    self.check_vector_data(name, self.ctypes[name], flat, dims[-1], line)
                 v = _Var(name, "data", dims, base, offset=len(self.blob), value=flat, orient=self.orients.get(name))
                 self.blob += flat
             else:
                 v = _Var(name, "data", [], base, value=(int(val) if base == "int" else float(val)))
             self.vars[name] = v
         # parameters block
-        off = 0
+        # parameters block: the density sees constrained values c[0 .. CDIM) (param leaves index them); a scalar
+        # coordinate has one of each, a simplex[K] K - 1 unconstrained coordinates and K constrained values
+        off, uoff = 0, 0
         for name, base, shape, lo, hi, init, line in self.blocks["parameters"]:
             if base != "real":
                 raise StanSubsetError(f"line {line}: parameters must be real")
@@ -1878,15 +2017,37 @@ class _Gen:
                                       f"column-major; declare an array of vectors)")
             v = _Var(name, "param", dims, "real", offset=off, lower=lov, upper=hiv, orient=self.orients.get(name))
             self.vars[name] = v
-            kind = "none" if (lov is None and hiv is None) else "both" if (lov is not None and hiv is not None) else \
-                "lower" if lov is not None else "upper"
             for j in range(v.size):
-                self.transforms.append((kind, lov, hiv))
                 self.param_names.append(name if not dims else f"{name}.{'.'.join(str(i + 1) for i in _unravel(j, dims))}")
+            kind = self.ctypes.get(name)
+            if kind is None:
+                kind = "none" if (lov is None and hiv is None) else "both" if (lov is not None and hiv is not None) else \
+                    "lower" if lov is not None else "upper"
+                for j in range(v.size):
+                    self.transforms.append((kind, lov, hiv))
+                    self.blocks_of.append((kind, lov, hiv, uoff + j, off + j, 1))
+                self.param_unc_names += self.param_names[len(self.param_names) - v.size:]
+                uoff += v.size
+            else:
+                K = dims[-1]
+                if K < (2 if kind == "simplex" else 1):
+                    raise StanSubsetError(f"line {line}: a {kind} needs at least {2 if kind == 'simplex' else 1} element(s)")
+                nu = K - 1 if kind == "simplex" else K
+                outer = dims[:-1]
+                for j in range(v.size // K):
+                    self.blocks_of.append((kind, None, None, uoff, off + j * K, K))
+                    for i in range(nu):
+                        self.transforms.append((kind, None, None))
+                        self.param_unc_names.append(f"{name}.{'.'.join(str(q + 1) for q in _unravel(j, outer) + [i])}"
+                                                    if outer else f"{name}.{i + 1}")
+                    uoff += nu
             off += v.size
-        self.dim = off
+        self.dim, self.cdim = uoff, off
         if not (1 <= self.dim <= self.MAX_DIM):
             raise StanSubsetError(f"{self.dim} unconstrained parameters; the generated kernels support 1..{self.MAX_DIM}")
+        if self.cdim > 2 * self.MAX_DIM:
+            raise StanSubsetError(f"{self.cdim} constrained parameter values; the generated kernels support up to "
+                                  f"{2 * self.MAX_DIM}")
         # transformed data (integer scalars folded now, everything else computed like a parameter-free local) and
         # transformed parameters (locals of the density; their declared bounds are validation only) run ahead of the model
         program = []
@@ -1923,32 +2084,72 @@ class _Gen:
         body = "\n".join(["        " + ln for ln in self.prologue] + self.lines[body_start:])
         return self.wrap(body)
 
+    @staticmethod
+    def check_vector_data(name, kind, flat, K, line):
+        """Stan validates constrained data when it reads it: rows of a simplex are >= 0 and sum to 1 (within 1e-8),
+        ordered rows increase strictly, positive_ordered rows also start above 0."""
+        for r in range(len(flat) // K):
+            row = flat[r * K:(r + 1) * K]
+            if kind == "simplex":
+                bad = any(not (z >= 0.0) for z in row) or not abs(math.fsum(row) - 1.0) <= 1e-8
+            else:
+                bad = any(not (b > a) for a, b in zip(row, row[1:])) or (kind == "positive_ordered" and not row[0] > 0.0)
+            if bad:
+                raise StanSubsetError(f"line {line}: data {name!r} is not a valid {kind} (row {r + 1}: {row})")
+
     def _const_value(self, e, line):
         n = self.real(e)
         if n.kind != "const":
             raise StanSubsetError(f"line {line}: parameter bounds must be constants")
         return n.val
 
+    _VECTOR_CALL = {"simplex": "simplex_{0}<{1}>", "ordered": "ordered_{0}<{1}, false>",
+                    "positive_ordered": "ordered_{0}<{1}, true>"}
+
     def wrap(self, body):
-        D = self.dim
-        pro = []
-        for k, (kind, lo, hi) in enumerate(self.transforms):
+        D, C = self.dim, self.cdim
+        pro, con, pull = [], [], []
+        for kind, lo, hi, u, k, K in self.blocks_of:
             if kind == "none":
-                pro.append(f"c[{k}] = x[{k}]; dc[{k}] = 1.0;")
+                pro.append(f"c[{k}] = x[{u}]; dc[{k}] = 1.0;")
+                con.append(f"out[{k}] = x[{u}];")
+                pull.append(f"g[{u}] = gc[{k}];")
             elif kind == "lower":
-                pro.append(f"{{ const double e = exp(x[{k}]); c[{k}] = {self.lit(lo)} + e; dc[{k}] = e; A += x[{k}]; gA[{k}] += 1.0; "
+                pro.append(f"{{ const double e = exp(x[{u}]); c[{k}] = {self.lit(lo)} + e; dc[{k}] = e; A += x[{u}]; gA[{k}] += 1.0; "
                            f"ok = ok && e > 0.0 && e < INFINITY; }}")
+                con.append(f"out[{k}] = {self.lit(lo)} + exp(x[{u}]);")
+                pull.append(f"g[{u}] = gc[{k}];")
             elif kind == "upper":
-                pro.append(f"{{ const double e = exp(x[{k}]); c[{k}] = {self.lit(hi)} - e; dc[{k}] = -e; A += x[{k}]; gA[{k}] += 1.0; "
+                pro.append(f"{{ const double e = exp(x[{u}]); c[{k}] = {self.lit(hi)} - e; dc[{k}] = -e; A += x[{u}]; gA[{k}] += 1.0; "
                            f"ok = ok && e > 0.0 && e < INFINITY; }}")
-            else:
+                con.append(f"out[{k}] = {self.lit(hi)} - exp(x[{u}]);")
+                pull.append(f"g[{u}] = gc[{k}];")
+            elif kind == "both":
                 w = self.lit(hi - lo)
-                pro.append(f"{{ const double s = smcgen_inv_logit(x[{k}]); c[{k}] = {self.lit(lo)} + {w} * s; dc[{k}] = {w} * s * (1.0 - s); "
+                pro.append(f"{{ const double s = smcgen_inv_logit(x[{u}]); c[{k}] = {self.lit(lo)} + {w} * s; dc[{k}] = {w} * s * (1.0 - s); "
                            f"A += log({w}) + log(s) + log1p(-s); gA[{k}] += 1.0 - 2.0 * s; ok = ok && s > 0.0 && s < 1.0; }}")
+                con.append(f"out[{k}] = {self.lit(lo)} + {w} * smcgen_inv_logit(x[{u}]);")
+                pull.append(f"g[{u}] = gc[{k}];")
+            else:        # a vector type: the body sees its K values as K independent leaves (dc = 1), pulled back below
+                fn = "smcb::stan::" + self._VECTOR_CALL[kind]
+                pro.append(f"A += {fn.format('constrain', K)}(&x[{u}], &c[{k}], ok);")
+                pro.append(f"for (int j = 0; j < {K}; ++j) dc[{k} + j] = 1.0;")
+                con.append(f"{fn.format('constrain', K)}(&x[{u}], &out[{k}], ok);")
+                pull.append(f"{fn.format('pullback', K)}(&x[{u}], " + (f"&c[{k}], " if kind == "simplex" else "")
+                            + f"&gc[{k}], &g[{u}]);")
+        if C == D and all(b[0] in ("none", "lower", "upper", "both") for b in self.blocks_of):
+            tail = f"""#pragma unroll
+        for (int k = 0; k < {D}; ++k) g[k] = gA[k] + phi * gB[k];"""
+        else:            # gradient over the constrained values, then one pullback per transform (log-Jacobian included)
+            tail = f"""double gc[{C}];
+#pragma unroll
+        for (int k = 0; k < {C}; ++k) gc[k] = gA[k] + phi * gB[k];
+        """ + "\n        ".join(pull)
         staged = len(self.blob) if len(self.blob) <= 4096 else 0
         text = f"""// GENERATED by smcnuts/model/stan_codegen.py -- do not edit.  Model struct with the interface of csrc/models.cuh.
 #pragma once
 #include <cmath>
+#include "stan_transforms.cuh"
 #ifndef SMCGEN_HELPERS
 #define SMCGEN_HELPERS
 SMCB_HD double smcgen_inv_logit(double z) {{ return z >= 0.0 ? 1.0 / (1.0 + exp(-z)) : exp(z) / (1.0 + exp(z)); }}
@@ -1964,7 +2165,7 @@ SMCB_HD double smcgen_digamma(double x) {{
 }}
 #endif
 struct {self.struct_name} {{
-    static constexpr int DMAX = {D}, STATIC_D = {D};
+    static constexpr int DMAX = {D}, STATIC_D = {D}, CDIM = {C};
     static constexpr int GROUP = 1, NLOC = {D}, STATIC_NL = {D};
     static constexpr bool STAGE = false;
     static constexpr int NDATA = {len(self.blob)}, NSTAGED = {staged};
@@ -1977,14 +2178,20 @@ struct {self.struct_name} {{
 
     // A = log prior + log Jacobian (everything not multiplied by phi), B = the phi-scaled part, g = grad A + phi * grad B
     SMCB_HD void eval(const double (&x)[DMAX], double phi, double& A_out, double& B_out, double (&g)[DMAX]) const {{
-        double A = 0.0, B = 0.0, gA[{D}] = {{0.0}}, gB[{D}] = {{0.0}}, c[{D}], dc[{D}];
+        double A = 0.0, B = 0.0, gA[{C}] = {{0.0}}, gB[{C}] = {{0.0}}, c[{C}], dc[{C}];
         bool ok = true;
         {(chr(10) + '        ').join(pro)}
 {body}
         if (!ok) A = -INFINITY;      // a constrained value under- or overflowed: Stan throws, the reference maps it to -inf
         A_out = A; B_out = B;
-#pragma unroll
-        for (int k = 0; k < {D}; ++k) g[k] = gA[k] + phi * gB[k];
+        {tail}
+    }}
+
+    // Stan's constraining transforms of the declared parameters, in declaration order: out[0 .. CDIM)
+    SMCB_HD static void constrain(const double (&x)[DMAX], double* out) {{
+        bool ok = true;
+        {(chr(10) + '        ').join(con)}
+        (void)ok;
     }}
 }};
 """
@@ -2026,7 +2233,7 @@ def generate(stan_text, data, struct_name="GenModel"):
     import hashlib
     parser = _Parser(stan_text)
     blocks = parser.program()
-    g = _Gen(blocks, data, struct_name, parser.orients)
+    g = _Gen(blocks, data, struct_name, parser.orients, parser.ctypes)
     text = g.run()
     digest = hashlib.sha256((text + repr(g.blob)).encode()).hexdigest()[:16]
-    return GeneratedSource(struct_name, text, g.dim, g.blob, g.param_names, g.transforms, digest)
+    return GeneratedSource(struct_name, text, g.dim, g.blob, g.param_names, g.transforms, digest, g.cdim, g.param_unc_names)

@@ -104,11 +104,13 @@ class SMCSampler:
             self._x_saved = self._logw_saved = None
         self._x_saved_host = self._logw_saved_host = None
 
-        self._mean_dev = dev.zeros(self.K + 1, D)
-        self._var_dev = dev.zeros(self.K + 1, D)
+        # estimates are on the constrained scale: a simplex[K] parameter has K - 1 coordinates in x but K columns here
+        DC = getattr(target, "constrained_dim", D)
+        self._mean_dev = dev.zeros(self.K + 1, DC)
+        self._var_dev = dev.zeros(self.K + 1, DC)
         self._moved = dev.zeros(self.K + 1)
-        self.mean_estimate = np.zeros([self.K + 1, D])
-        self.variance_estimate = np.zeros([self.K + 1, D])
+        self.mean_estimate = np.zeros([self.K + 1, DC])
+        self.variance_estimate = np.zeros([self.K + 1, DC])
 
     # History under the reference's names (smc_sampler.py:73-74): host NumPy arrays [K+1, N, D] / [K+1, N], materialised
     # lazily from the device-resident history on first access and cached (this rank's shard when particles are sharded).
