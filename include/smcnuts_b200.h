@@ -63,6 +63,15 @@ int smcb_model_dim(void* handle);
  * smcb_model_constrain writes out[N, CDIM] row-major (device) from the unconstrained rows x[N, dim] (device), on stream. */
 int smcb_model_constrained_dim(void* handle);
 int smcb_model_constrain(void* handle, const double* x, long long N, double* out, void* stream);
+/* Generated quantities of a plug-in model (the Stan program's `generated quantities` block, which BridgeStan's
+ * param_constrain(include_gq=True) appends).  smcb_model_gq_dim returns the row width G (0 for a built-in model or a program
+ * without the block).  smcb_model_generated_quantities writes out[N, G] row-major (device) from the unconstrained rows
+ * x[N, dim] (device), on stream; nothing when G = 0.  Row i draws its _rng values from the Philox stream 6 of
+ * (seed, counter, particle0 + i) -- global particle indices, so a particle's draws do not depend on how the rows are
+ * batched; counter < 2^24.  A row whose draws get invalid arguments (Stan throws) is NaN throughout. */
+int smcb_model_gq_dim(void* handle);
+int smcb_model_generated_quantities(void* handle, const double* x, long long N, uint64_t seed, uint32_t counter,
+                                    long long particle0, double* out, void* stream);
 /* Host-only test hook (no GPU work): the tensor-core fragment packing of the PRMwCD NUTS kernel (csrc/models.cuh,
  * PrmModelG) applied to a scalar blob [16 header doubles][n_obs rows of 12]; host_out gets 32 + tiles*288 doubles. */
 int smcb_debug_pack_prm(const double* host_scalar_blob, int n_obs, int tiles, double* host_out, long long n_out);

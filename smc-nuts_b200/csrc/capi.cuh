@@ -46,7 +46,7 @@ inline int check_launch(const char* where) {
 
 // Entry points of a generated model plug-in (nuts_plugin.cuh), resolved by smcb_model_create_plugin; a plug-in built
 // against another version of this table is refused
-#define SMCB_PLUGIN_ABI 2
+#define SMCB_PLUGIN_ABI 3
 struct NutsArgs;
 struct PluginVT {
     void* dl;
@@ -59,6 +59,8 @@ struct PluginVT {
     int (*logp_grad)(const ModelDesc*, const double*, long long, double, double*, double*, double*, void*);
     int (*constrained_dim)(void);
     int (*constrain)(const ModelDesc*, const double*, long long, double*, void*);
+    int (*gq_dim)(void);
+    int (*generated_quantities)(const ModelDesc*, const double*, long long, uint64_t, uint32_t, long long, double*, void*);
 };
 
 struct Model {

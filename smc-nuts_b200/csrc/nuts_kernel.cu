@@ -120,6 +120,9 @@ int smcb_model_create_plugin(const char* so_path, const double* host_data, long 
     vt->logp_grad = (int (*)(const ModelDesc*, const double*, long long, double, double*, double*, double*, void*))sym("smcb_plugin_logp_grad");
     vt->constrained_dim = (int (*)(void))sym("smcb_plugin_constrained_dim");
     vt->constrain = (int (*)(const ModelDesc*, const double*, long long, double*, void*))sym("smcb_plugin_constrain");
+    vt->gq_dim = (int (*)(void))sym("smcb_plugin_gq_dim");
+    vt->generated_quantities = (int (*)(const ModelDesc*, const double*, long long, uint64_t, uint32_t, long long, double*,
+                                        void*))sym("smcb_plugin_generated_quantities");
     auto bail = [&](const char* what) { dlclose(dl); delete vt; return fail("smcb_model_create_plugin", what); };
     if (!ok) return bail("not a model plug-in: an smcb_plugin_* entry point is missing (csrc/nuts_plugin.cuh)");
     if (vt->abi() != SMCB_PLUGIN_ABI) return bail("plug-in ABI version mismatch: rebuild it against this library's csrc/");
@@ -185,6 +188,25 @@ int smcb_model_constrain(void* handle, const double* x, long long N, double* out
     if (N == 0) return 0;
     const Model* m = (const Model*)handle;
     if (m->vt->constrain(&m->desc, x, N, out, stream)) return fail("smcb_model_constrain (plug-in)", m->vt->last_error());
+    g_launches.fetch_add(1, std::memory_order_relaxed);
+    return 0;
+}
+
+int smcb_model_gq_dim(void* handle) {
+    SMCB_REQUIRE(handle, "null argument");
+    const Model* m = (const Model*)handle;
+    return m->vt ? m->vt->gq_dim() : 0;
+}
+
+int smcb_model_generated_quantities(void* handle, const double* x, long long N, uint64_t seed, uint32_t counter,
+                                    long long particle0, double* out, void* stream) {
+    SMCB_REQUIRE(handle && N >= 0 && particle0 >= 0, "bad argument");
+    SMCB_REQUIRE(counter < (1u << 24), "bad argument: the call counter has 24 bits");
+    const Model* m = (const Model*)handle;
+    if (!m->vt || N == 0 || m->vt->gq_dim() == 0) return 0;
+    SMCB_REQUIRE(x && out, "bad argument");
+    if (m->vt->generated_quantities(&m->desc, x, N, seed, counter, particle0, out, stream))
+        return fail("smcb_model_generated_quantities (plug-in)", m->vt->last_error());
     g_launches.fetch_add(1, std::memory_order_relaxed);
     return 0;
 }

@@ -18,7 +18,8 @@ enum Stream : uint32_t {
     kStreamAccRej = 2,    // endpoint MH uniform                    (utils.py:32)
     kStreamResample = 3,  // resampling uniforms (particle = slot)  (samples.py:139)
     kStreamInit = 4,      // x0 ~ N(0, I)                           (samples.py:77)
-    kStreamEstimate = 5   // estimate_from_tempered resampling      (estimate_from_tempered.py:43)
+    kStreamEstimate = 5,  // estimate_from_tempered resampling      (estimate_from_tempered.py:43)
+    kStreamGQ = 6         // _rng draws of generated quantities     (stan_rng.cuh)
 };
 
 struct Philox4 {

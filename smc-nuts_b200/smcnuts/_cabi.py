@@ -10,7 +10,7 @@ LIB_PATH = Path(os.environ.get("SMCB_LIB_PATH") or (_PKG / "_lib" / "libsmcnuts_
 HEADER = _PKG.parents[1] / "include" / "smcnuts_b200.h"
 
 MODEL_KINDS = {"arma": 0, "PRMwCD": 1, "gauss": 2}
-STREAM_NUTS, STREAM_MOMENTUM, STREAM_ACCREJ, STREAM_RESAMPLE, STREAM_INIT, STREAM_ESTIMATE = range(6)
+STREAM_NUTS, STREAM_MOMENTUM, STREAM_ACCREJ, STREAM_RESAMPLE, STREAM_INIT, STREAM_ESTIMATE, STREAM_GQ = range(7)
 CONSTRAIN_NONE, CONSTRAIN_EXP_LAST = 0, 1
 CONSTRAIN_MODEL = 2   # host side only: constrain through the model (smcb_model_constrain) first, then unconstrained moments
 
@@ -26,6 +26,8 @@ _SIGS = {
     "smcb_model_dim": [_vp],
     "smcb_model_constrained_dim": [_vp],
     "smcb_model_constrain": [_vp, _vp, _ll, _vp, _vp],
+    "smcb_model_gq_dim": [_vp],
+    "smcb_model_generated_quantities": [_vp, _vp, _ll, _u64, _u32, _ll, _vp, _vp],
     "smcb_debug_pack_prm": [_vp, _i, _i, _vp, _ll],
     "smcb_logp_grad": [_vp, _vp, _ll, _d, _vp, _vp, _vp, _vp],
     "smcb_combine_logp": [_vp, _vp, _d, _ll, _vp, _vp],

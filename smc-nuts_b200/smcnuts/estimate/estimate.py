@@ -7,6 +7,8 @@ the shipped models) is fused into the moment kernel instead of N BridgeStan call
 from .. import _cabi, _device as dev
 from ..parallel import ShardContext
 
+MOMENT_COLS = 256     # widest row smcb_weighted_moment reduces in one launch
+
 
 class Estimate:
     def __init__(self, target, shard: ShardContext = None):
@@ -42,6 +44,19 @@ class Estimate:
         if constrain == _cabi.CONSTRAIN_MODEL:     # generated models: [N, dim] -> [N, constrained_dim] through the plug-in
             xd, constrain = self.target.constrain(xd), _cabi.CONSTRAIN_NONE
         N, D = xd.shape
+        if D > MOMENT_COLS:      # wide rows (generated quantities): column blocks, the exp-on-last in the last one only
+            mean, var = dev.empty(D), dev.empty(D)
+            for j in range(0, D, MOMENT_COLS):
+                k = min(j + MOMENT_COLS, D)
+                m, v = self._moments(xd[:, j:k].contiguous(), wd, constrain if k == D else _cabi.CONSTRAIN_NONE)
+                mean[j:k].copy_(m)
+                var[j:k].copy_(v)
+        else:
+            mean, var = self._moments(xd, wd, constrain)
+        return dev.like_input(mean, x), dev.like_input(var, x)
+
+    def _moments(self, xd, wd, constrain):
+        N, D = xd.shape
         mean, var = dev.empty(D), dev.empty(D)
         ws, st = dev.reduce_ws(), dev.stream_ptr()
         _cabi.call("smcb_weighted_moment", dev.ptr(xd), dev.ptr(wd), N, D, constrain, 0, 1, dev.ptr(mean),
@@ -50,4 +65,4 @@ class Estimate:
         _cabi.call("smcb_weighted_moment", dev.ptr(xd), dev.ptr(wd), N, D, constrain, dev.ptr(mean), 2, dev.ptr(var),
                    dev.ptr(ws), st)
         self.shard.all_reduce_sum_(var)
-        return dev.like_input(mean, x), dev.like_input(var, x)
+        return mean, var

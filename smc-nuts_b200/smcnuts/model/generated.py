@@ -4,7 +4,8 @@ The reference compiles arbitrary Stan programs through BridgeStan (smcnuts/model
 `stan_codegen.generate` translates the program into a model struct, this module wraps it into a plug-in translation
 unit (csrc/nuts_plugin.cuh), compiles it with nvcc for sm_100a into smcnuts/_lib/gen/<digest>/model.so and hands it to
 the library with smcb_model_create_plugin.  The result has the reference's target API (`dim`, `constrained_dim`,
-`param_names`, `logpdf`, `logpdfgrad`, `constrain`) and runs through the same NUTS / SMC kernels as the built-in models.
+`param_names`, `logpdf`, `logpdfgrad`, `constrain`) and runs through the same NUTS / SMC kernels as the built-in models;
+`generated_quantities` (with `gq_dim`, `gq_names`) evaluates the program's generated quantities block at particles.
 No CPU fallback: without nvcc or a GPU the constructor raises.
 """
 import ctypes
@@ -52,17 +53,18 @@ def build_plugin(src: stan_codegen.GeneratedSource, force=False, parity=False):
     work = Path(tempfile.mkdtemp(prefix=out_dir.name + ".", dir=GEN_DIR))
     try:
         (work / "model_gen.cuh").write_text(src.text)
+        (work / "model_gq.cuh").write_text(src.gq_text)
         (work / "plugin.cu").write_text(
             "// GENERATED: plug-in translation unit of a Stan-subset model (smcnuts/model/generated.py)\n"
-            "#define SMCB_PLUGIN_TU 1\n#include \"nuts_plugin.cuh\"\n#include \"model_gen.cuh\"\n"
-            f"SMCB_DEFINE_PLUGIN({src.struct_name})\n")
+            "#define SMCB_PLUGIN_TU 1\n#include \"nuts_plugin.cuh\"\n#include \"model_gen.cuh\"\n#include \"model_gq.cuh\"\n"
+            f"SMCB_DEFINE_PLUGIN({src.struct_name})\nSMCB_DEFINE_PLUGIN_GQ({src.struct_name}GQ)\n")
         flags = NVCC_FLAGS + (["-DSMCB_PARITY=1", "-fmad=false"] if parity else [])
         cmd = [nvcc, *flags, f"-I{CSRC}", f"-I{work}", str(work / "plugin.cu"), "-o", str(work / "model.so")]
         r = subprocess.run(cmd, capture_output=True, text=True)
         if r.returncode != 0:
             raise _cabi.SmcbError(f"nvcc failed for the generated model:\n{r.stdout}\n{r.stderr}")
         out_dir.mkdir(parents=True, exist_ok=True)
-        for name in ("model_gen.cuh", "plugin.cu"):
+        for name in ("model_gen.cuh", "model_gq.cuh", "plugin.cu"):
             os.replace(work / name, out_dir / name)
         os.replace(work / "model.so", so)          # last: its presence marks the directory as complete
     finally:
@@ -92,6 +94,10 @@ class GeneratedModel(DeviceModel):
         # are skipped (generated quantities) but are NOT appended: estimates cover the declared parameters only
         self.constrained_dim = _cabi.lib().smcb_model_constrained_dim(self._h)
         assert self.constrained_dim == self.source.cdim, (self.constrained_dim, self.source.cdim)
+        # generated quantities: a separate output of gq_dim columns (gq_names in BridgeStan's form); 0 without the block
+        self.gq_names = list(self.source.gq_names)
+        self.gq_dim = _cabi.lib().smcb_model_gq_dim(self._h)
+        assert self.gq_dim == self.source.gq_dim, (self.gq_dim, self.source.gq_dim)
         kinds = [t[0] for t in self.source.transforms]
         if all(k == "none" for k in kinds):
             self.constrain_kind = _cabi.CONSTRAIN_NONE
@@ -112,6 +118,23 @@ class GeneratedModel(DeviceModel):
         out = dev.empty(xd.shape[0], self.constrained_dim)
         _cabi.call("smcb_model_constrain", self._h, dev.ptr(xd), xd.shape[0], dev.ptr(out), dev.stream_ptr())
         shape = tuple(np.shape(x)[:-1]) + (self.constrained_dim,)
+        if dev.is_host(x):
+            return dev.to_numpy(out).reshape(shape)
+        return out.reshape(shape)
+
+    def generated_quantities(self, x, seed=None, counter=0, particle0=0):
+        """The program's generated quantities at the particles x: [..., dim] -> [..., gq_dim], one kernel of the model's
+        plug-in (host in -> host out, device in -> device out).  The _rng draws of row i come from the Philox stream of
+        (seed, counter, particle0 + i): the same particle index, seed and counter give the same draws in any batch
+        (seed None -> 0; counter < 2^24).  Rows whose draws get invalid arguments are NaN.  Raises the generator's
+        StanSubsetError when the block is outside the supported subset."""
+        if self.source.gq_error is not None:
+            raise stan_codegen.StanSubsetError(f"generated quantities: {self.source.gq_error}")
+        xd = dev.to_device(x).reshape(-1, self.dim).contiguous()
+        out = dev.empty(xd.shape[0], self.gq_dim)
+        _cabi.call("smcb_model_generated_quantities", self._h, dev.ptr(xd), xd.shape[0], dev.seed_from_rng(seed), int(counter),
+                   int(particle0), dev.ptr(out), dev.stream_ptr())
+        shape = tuple(np.shape(x)[:-1]) + (self.gq_dim,)
         if dev.is_host(x):
             return dev.to_numpy(out).reshape(shape)
         return out.reshape(shape)

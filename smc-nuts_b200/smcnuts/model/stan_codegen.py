@@ -27,8 +27,8 @@ What is generated
 
 Supported subset (anything else raises StanSubsetError with the offending line):
   blocks functions (functions returning real, inlined at the call: no recursion, one return at the end) / data /
-  transformed data / parameters / transformed parameters / model (generated quantities is skipped: it never enters the
-  log density);  int, real, vector, row_vector, matrix (data and
+  transformed data / parameters / transformed parameters / model / generated quantities (below);  int, real, vector,
+  row_vector, matrix (data and
   locals), array[..] (and the pre-2.33 `real y[N]` form);  lower/upper bounds on real parameters;  simplex[K], ordered[K],
   positive_ordered[K] (and arrays of them) as parameters, as data (validated at generation time: rows >= 0 summing to 1
   within 1e-8, strictly increasing) and as plain vectors in transformed parameters;  local declarations
@@ -47,6 +47,19 @@ Supported subset (anything else raises StanSubsetError with the offending line):
   scalar or vectorised over container arguments and container-valued argument expressions;  dirichlet (alpha data or
   parameters), categorical (an int or int array outcome) and multinomial (an int array) of a vector argument, the integer
   outcomes being data known at generation time (tabulated into counts).
+
+Generated quantities (a separate output: `constrain()`, `param_names` and the density code do not change)
+  a second struct `<struct_name>GQ` (GeneratedSource.gq_text) with generated_quantities(x, rng, out): value-only code
+  (no sensitivities, no A / B split) of transformed data, transformed parameters and the block, over the constrained
+  parameters; the outputs are the block's top-level int / real / vector / row_vector declarations and arrays of them
+  (gq_names: BridgeStan's name.i.j, ints written as doubles).  Every construct of the model block is accepted, densities
+  by value (`normal_lpdf(y[n] | mu[n], sigma)`), plus the _rng functions of csrc/stan_rng.cuh: normal, std_normal,
+  student_t, cauchy, double_exponential, logistic, lognormal, exponential, gamma, inv_gamma, beta, uniform, bernoulli,
+  bernoulli_logit, binomial, poisson, poisson_log, neg_binomial_2 (scalar, or vectorised into arrays) and categorical (of a
+  vector).  `target +=`, `~`, phi and redeclared names are refused there, _rng calls everywhere else; G is at most
+  MAX_GQ (one row of a particle block fits in shared memory).  A block outside this subset does
+  not stop the model: its StanSubsetError text (with the line) is kept in GeneratedSource.gq_error and raised when gq
+  values are requested.
 """
 import json
 import math
@@ -95,6 +108,7 @@ class _Parser:
         self.i = 0
         self.orients = {}       # variable name -> "col" (vector) | "row" (row_vector) | "mat" (matrix): how `*` treats it
         self.ctypes = {}        # variable name -> "simplex" | "ordered" | "positive_ordered"
+        self.gq_orients, self.gq_ctypes = {}, {}    # the same, with the declarations of generated quantities added
 
     def peek(self, k=0):
         return self.t[self.i + k]
@@ -135,16 +149,22 @@ class _Parser:
                 while self.peek()[1] != "}":
                     fname, fn = self.function()
                     blocks[name][fname] = fn
+            elif name == "generated quantities":
+                # parsed with orientations / vector kinds of its own (the density code must not see its declarations);
+                # a block outside the subset is kept as its error: the density does not need it
+                start, saved = self.i, (dict(self.orients), dict(self.ctypes))
+                try:
+                    blocks[name] = self.stmts()
+                except StanSubsetError as e:
+                    blocks["generated quantities error"] = str(e)
+                    self.i = start
+                    self.skip_block()
+                    continue
+                finally:
+                    self.gq_orients, self.gq_ctypes = self.orients, self.ctypes
+                    self.orients, self.ctypes = saved
             else:
-                depth, empty = 1, True
-                while depth:
-                    tok = self.next()
-                    depth += (tok[1] == "{") - (tok[1] == "}")
-                    empty = empty and tok[1] == "}"
-                    if tok[0] == "eof":
-                        self.err("unterminated block")
-                # generated quantities never enter the log density (bridgestan.py:60-85 only calls log_density*): skipped
-                if not empty and name != "generated quantities":
+                if not self.skip_block():
                     raise StanSubsetError(f"block {name!r} is outside the supported subset")
                 continue
             self.expect("}")
@@ -153,6 +173,17 @@ class _Parser:
                 raise StanSubsetError(f"missing block {need!r}")
         blocks.setdefault("data", [])
         return blocks
+
+    def skip_block(self):
+        """Skips to the `}` that closes the current block (consumed) -> whether the block was empty."""
+        depth, empty = 1, True
+        while depth:
+            tok = self.next()
+            depth += (tok[1] == "{") - (tok[1] == "}")
+            empty = empty and tok[1] == "}"
+            if tok[0] == "eof":
+                self.err("unterminated block")
+        return empty
 
     # ---- user-defined functions: name -> (return type, [(argument name, kind)], body statements, line);  kind is "int",
     #      "real" or "container" (vector / row_vector / array: bound by name at the call)
@@ -600,6 +631,18 @@ def _sum_exprs(terms, line):
     return out
 
 
+# _rng functions of generated quantities (csrc/stan_rng.cuh) -> number of arguments
+_RNG_ARITY = {"normal": 2, "std_normal": 0, "student_t": 3, "cauchy": 2, "double_exponential": 2, "logistic": 2,
+              "lognormal": 2, "exponential": 1, "gamma": 2, "inv_gamma": 2, "beta": 2, "uniform": 2, "bernoulli": 1,
+              "bernoulli_logit": 1, "binomial": 2, "poisson": 1, "poisson_log": 1, "neg_binomial_2": 2, "categorical": 1}
+
+
+def _has_rng(e):
+    found = []
+    _walk_exprs(e, lambda x: found.append(x) if x[0] == "call" and str(x[1]).endswith("_rng") else None)
+    return bool(found)
+
+
 _UNARY_FUNCS = {"exp": "exp", "log": "log", "log1p": "log1p", "sqrt": "sqrt", "fabs": "fabs", "abs": "fabs", "lgamma": "lgamma",
                 "tanh": "tanh", "sin": "sin", "cos": "cos", "inv_logit": "inv_logit", "log1p_exp": "log1p_exp"}
 
@@ -809,20 +852,29 @@ class _Var:
 class GeneratedSource:
     """Result of `generate`: C++ text of the model struct and what the host side needs to know about it."""
 
-    def __init__(self, struct_name, text, dim, blob, param_names, transforms, digest, cdim, param_unc_names):
+    def __init__(self, struct_name, text, dim, blob, param_names, transforms, digest, cdim, param_unc_names,
+                 gq_text="", gq_names=(), gq_error=None):
         self.struct_name, self.text, self.dim, self.blob = struct_name, text, dim, blob
         self.param_names, self.transforms, self.digest = param_names, transforms, digest
         self.cdim, self.param_unc_names = cdim, param_unc_names      # constrained width, unconstrained names
+        # generated quantities: the struct `<struct_name>GQ` (included after `text`), its output names in BridgeStan's
+        # form, and -- for a block outside the subset -- the StanSubsetError text, raised when gq values are requested
+        self.gq_text, self.gq_names, self.gq_error = gq_text, list(gq_names), gq_error
+        self.gq_dim = len(self.gq_names)
 
 
 class _Gen:
     MAX_DIM = 64
+    MAX_GQ = 24576          # outputs of generated quantities: a row of a particle block fits in shared memory
 
-    def __init__(self, blocks, data, struct_name, orients=None, ctypes=None):
+    def __init__(self, blocks, data, struct_name, orients=None, ctypes=None, value_only=False):
         self.blocks, self.struct_name = blocks, struct_name
+        self.value_only = value_only    # generated quantities: values only (no sensitivities, no A / B split), _rng calls
         self.orients = orients or {}
         self.ctypes = ctypes or {}
         self.lowered = {}       # id(statement) -> its scalar-subset replacement (list of statements) or None
+        self.rng_stmts = {}     # id(statement) -> the statement with its draws ahead of it, or None (value-only mode)
+        self.scopes = [set()]   # value-only mode: names declared in each enclosing scope (Stan refuses redeclarations)
         self.fresh = 0
         self.functions = blocks.get("functions", {})
         self.inline_depth = 0
@@ -949,6 +1001,8 @@ class _Gen:
 
     def call(self, e):
         name, args, line = e[1], e[2], e[3]
+        if name.endswith("_rng"):
+            return self.rng_call(name, args, line)
         m = re.fullmatch(r"(\w+?)_(lpdf|lpmf|log)", name)
         if m and m.group(1) in _DENSITIES:
             return _add(*self.density_terms(m.group(1), args, line, vectorised=False))
@@ -967,6 +1021,23 @@ class _Gen:
             return _add(a, _un("log1p_exp", _sub(b, a)))
         raise StanSubsetError(f"line {line}: function {name!r} is outside the supported subset")
 
+    def rng_call(self, name, args, line):
+        """One draw of a scalar _rng function (csrc/stan_rng.cuh); categorical_rng takes a whole vector variable."""
+        if not self.value_only:
+            raise StanSubsetError(f"line {line}: {name}: _rng functions are only allowed in generated quantities")
+        dist = name[:-4]
+        if dist not in _RNG_ARITY:
+            raise StanSubsetError(f"line {line}: function {name!r} is outside the supported subset")
+        if len(args) != _RNG_ARITY[dist]:
+            raise StanSubsetError(f"line {line}: {name} takes {_RNG_ARITY[dist]} argument(s)")
+        if dist == "categorical":
+            v = self.vars.get(args[0][1]) if args[0][0] == "var" else None
+            if v is None or len(v.shape) != 1:
+                raise StanSubsetError(f"line {line}: categorical_rng takes a vector")
+            ptr = {"data": f"&data[{v.offset}]", "param": f"&c[{v.offset}]"}.get(v.kind, f"v_{v.name}")
+            return Node("rng", op=dist, name=ptr, idx=v.shape[0])
+        return Node("rng", op=dist, args=tuple(self.real(a) for a in args))
+
     def density_terms(self, dist, args, line, vectorised=True):
         fn = _DENSITIES[dist]
         if len(args) != fn.__code__.co_argcount:
@@ -975,7 +1046,10 @@ class _Gen:
 
     def hoist_lgamma(self, n):
         """lgamma(data[i] + c) is tabulated at generation time as one more data array (the log-factorials of a count
-        likelihood would otherwise be a run-time lgamma per observation and evaluation)."""
+        likelihood would otherwise be a run-time lgamma per observation and evaluation).  Generated quantities read the
+        density's data blob as it is: there lgamma runs per evaluation."""
+        if self.value_only:
+            return n
         if n.kind not in ("un", "bin") or n.deps:
             if n.kind in ("un", "bin"):
                 args = tuple(self.hoist_lgamma(a) for a in n.args)
@@ -1082,10 +1156,14 @@ class _Gen:
                 if n is None:
                     raise StanSubsetError(f"line {e[3]}: the size of {name} must be a constant")
                 return (n,), {"rep_vector": "col", "rep_row_vector": "row", "rep_array": None}[name]
+            if name == "categorical_rng":
+                return (), None
             shapes = [self.shape(a) for a in args]
             big = [sh for sh in shapes if sh[0]]
             if big and any(sh[0] != big[0][0] for sh in big):
                 raise StanSubsetError(f"line {e[3]}: arguments of {name} have different sizes")
+            if big and name.endswith("_rng"):       # vectorised draws are arrays, as in Stan
+                return big[0][0], None
             return big[0] if big else ((), None)
         raise StanSubsetError(f"unsupported expression {e!r}")
 
@@ -1155,6 +1233,16 @@ class _Gen:
                 return ("bin", "/", total, ("num", float(n), False)) if name == "mean" else total
             if name in self.functions:
                 return self.lower(self.inline(name, args, pre, cl), [], pre, cl)
+            if name == "categorical_rng" and len(args) == 1 and args[0][0] != "var":   # the vector is materialised first
+                dims, orient = self.shape(args[0])
+                if len(dims) != 1:
+                    raise StanSubsetError(f"line {cl}: categorical_rng takes a vector")
+                tmp = self.fresh_name("theta")
+                self.vars[tmp] = _Var(tmp, "local", list(dims), "real", orient=orient)
+                pre.append(("decl", (tmp, "real", [("num", float(dims[0]), True)], None, None, args[0], cl), cl))
+                return ("call", name, [("var", tmp, cl)], cl)
+            if name == "categorical_rng":
+                return e
             if name == "log_sum_exp" and len(args) == 1:
                 return self.log_sum_exp(args[0], pre, cl)
             m = re.fullmatch(r"(\w+?)_(lpdf|lpmf|log)", name)
@@ -1680,6 +1768,13 @@ class _Gen:
                 name[id(n)] = f"data[{n.idx}]"
             elif n.kind == "ivar":
                 name[id(n)] = f"(double){n.name}"
+            elif n.kind == "rng":       # a draw: never shared between evaluations, never hoisted
+                a = [name[id(x)] for x in n.args] + ["rng"]
+                fn = f"categorical_rng<{n.idx}>" if n.op == "categorical" else f"{n.op}_rng"
+                t = self.new_tmp()
+                self.emit(f"const double {t} = smcb::stan::{fn}({n.name + ', ' if n.op == 'categorical' else ''}"
+                          f"{', '.join(a)});")
+                name[id(n)] = t
             else:
                 a = [name[id(x)] for x in n.args]
                 if n.kind == "un":
@@ -1698,6 +1793,8 @@ class _Gen:
                 t = self.new_tmp()
                 self.emit(f"const double {t} = {text};")
                 name[id(n)] = t
+        if self.value_only:
+            return name[id(root)], []
         # reverse sweep over the nodes that depend on parameters
         adj = {id(root): ["1.0"]}
         leaves = []
@@ -1854,7 +1951,9 @@ class _Gen:
         self.emit("{")
         self.indent += 1
         val, leaves = self.emit_value_and_adjoints(rhs_node)
-        if op == "=":
+        if self.value_only:
+            self.emit(f"{cell} {op} {val};")
+        elif op == "=":
             reads_self = any(n.kind == "local" and n.name == v.name for n, _ in leaves)
             if reads_self and v.deps:        # the old sensitivities are inputs: build the new ones aside
                 self.emit(f"double nd[{max(v.deps) + 1}];")
@@ -1873,9 +1972,66 @@ class _Gen:
         self.indent -= 1
         self.emit("}")
 
+    def hoist_rng(self, e, pre, line, top=False):
+        """`e` with every _rng call below it (innermost first; `top`: not `e` itself) replaced by a fresh local that a
+        declaration appended to `pre` draws into: each call is evaluated once, as Stan does, however often the lowering
+        reads the expression."""
+        if isinstance(e, list):
+            return [self.hoist_rng(x, pre, line) for x in e]
+        if not (isinstance(e, tuple) and e and isinstance(e[0], str)) or not _has_rng(e):
+            return e
+        if e[0] != "call":
+            return tuple(self.hoist_rng(x, pre, line) if isinstance(x, (tuple, list)) else x for x in e)
+        new = ("call", e[1], [self.hoist_rng(a, pre, line) for a in e[2]], e[3])
+        if top or not e[1].endswith("_rng"):
+            return new
+        dims, orient = self.shape(new)
+        tmp = self.fresh_name("draw")
+        self.vars[tmp] = _Var(tmp, "local", list(dims), "real", orient=orient)
+        pre.append(("decl", (tmp, "real", [("num", float(d), True) for d in dims], None, None, new, line), line))
+        return ("var", tmp, line)
+
+    def hoist_rng_stmt(self, s):
+        """Value-only mode: the statement with its _rng calls drawn ahead of it (a list), or None when it has nothing to
+        draw first; cached by identity like lower_stmt."""
+        key = id(s)
+        if key not in self.rng_stmts:
+            kind, line, out, pre = s[0], s[-1], None, []
+            if kind in ("if", "while") and _has_rng(s[1]):
+                raise StanSubsetError(f"line {line}: _rng calls inside a condition are outside the supported subset "
+                                      f"(draw into a variable first)")
+            if kind == "assign" and _has_rng(s):
+                rhs = self.hoist_rng(s[3], pre, line, top=True)
+                lhs = self.hoist_rng(s[1], pre, line)
+                out = pre + [("assign", lhs, s[2], rhs, line)] if pre else None
+            elif kind == "decl" and s[1][5] is not None and _has_rng(s[1][5]):
+                d = s[1]
+                init = self.hoist_rng(d[5], pre, line, top=True)
+                out = pre + [("decl", (d[0], d[1], d[2], d[3], d[4], init, d[6]), line)] if pre else None
+            self.rng_stmts[key] = (s, out)
+        return self.rng_stmts[key][1]
+
+    def scoped(self, stmts, emit):
+        """statements() of a nested scope: a block, a loop body or a branch (value-only mode tracks its declarations)"""
+        if not self.value_only:
+            self.statements(stmts, emit)
+            return
+        self.scopes.append(set())
+        try:
+            self.statements(stmts, emit)
+        finally:
+            self.scopes.pop()
+
     def statements(self, stmts, emit=True):
         for s in stmts:
             kind, line = s[0], s[-1]
+            if self.value_only:
+                if kind in ("target", "tilde", "ptarget"):
+                    raise StanSubsetError(f"line {line}: `target +=` and `~` are only allowed in the model block")
+                drawn = self.hoist_rng_stmt(s)
+                if drawn is not None:
+                    self.statements(drawn, emit)
+                    continue
             low = self.lower_stmt(s)
             if low is not None:
                 self.statements(low, emit)
@@ -1887,13 +2043,13 @@ class _Gen:
                     self.indent += 1
                     self.emit(f"if ({self.cond_text(cond, line)}) {{")
                     self.indent += 1
-                self.statements([then], emit)
+                self.scoped([then], emit)
                 if other is not None:
                     if emit:
                         self.indent -= 1
                         self.emit("} else {")
                         self.indent += 1
-                    self.statements([other], emit)
+                    self.scoped([other], emit)
                 if emit:
                     self.indent -= 1
                     self.emit("}")
@@ -1913,7 +2069,7 @@ class _Gen:
                     self.indent += 1
                     self.emit(f"if ({trip} >= (1 << 24)) {{ ok = false; break; }}")
                     self.emit(f"if (!{self.cond_text(s[1], line)}) break;")
-                self.statements([s[2]], emit)
+                self.scoped([s[2]], emit)
                 if emit:
                     self.indent -= 1
                     self.emit("}")
@@ -1922,6 +2078,10 @@ class _Gen:
                 name, base, shape, lo, hi, init, _ = s[1]
                 if name in self.vars and self.vars[name].kind != "local":
                     raise StanSubsetError(f"line {line}: {name!r} shadows a data variable or parameter")
+                if self.value_only:
+                    if any(name in sc for sc in self.scopes):
+                        raise StanSubsetError(f"line {line}: {name!r} is already declared")
+                    self.scopes[-1].add(name)
                 dims = []
                 for d in shape:
                     dv, _ = self.int_expr(d)
@@ -1934,7 +2094,7 @@ class _Gen:
                     first = self.decl_init.setdefault(id(s), ("assign", ("var", name, line), "=", init, line))
                     self.statements([first], emit)
             elif kind == "block":
-                self.statements(s[1], emit)
+                self.scoped(s[1], emit)
             elif kind == "for":
                 _, var, lo, hi, body, _ = s
                 (lov, loc), (hiv, hic) = self.int_expr(lo), self.int_expr(hi)
@@ -1946,7 +2106,7 @@ class _Gen:
                     self.emit(f"for (int {cname} = {loc}; {cname} <= {hic}; ++{cname}) {{")
                     self.indent += 1
                 self.loop_vars.append((var, cname))
-                self.statements(body, emit)
+                self.scoped(body, emit)
                 self.loop_vars.pop()
                 if emit:
                     self.indent -= 1
@@ -1980,6 +2140,63 @@ class _Gen:
 
     # ---- driver
     def run(self):
+        # transformed data and transformed parameters (locals of the density; their declared bounds are validation only)
+        # run ahead of the model
+        program = self.declare_inputs()
+        program += self.blocks.get("transformed parameters", [])
+        program += self.blocks["model"]
+        self.blocks["model"] = _demote_arrays(self.fuse_vector_densities(program)) if RESTRUCTURE else program
+        # activity analysis (which coordinates can each local depend on): fixpoint over the statement list
+        for _ in range(64):
+            self.changed = False
+            self.loop_vars = []
+            self.statements(self.blocks["model"], emit=False)
+            if not self.changed:
+                break
+        # emission
+        self.loop_vars = []
+        body_start = len(self.lines)
+        for v in self.vars.values():
+            if v.kind == "local":
+                dims = "".join(f"[{n}]" for n in ([v.size] if v.shape else []))
+                self.emit(f"double v_{v.name}{dims}{' = {0.0}' if v.shape else ' = 0.0'};")
+                if v.deps:
+                    self.emit(f"double d_{v.name}{dims}[{max(v.deps) + 1}]{' = {{0.0}}' if v.shape else ' = {0.0}'};")
+        self.statements(self.blocks["model"], emit=True)
+        body = "\n".join(["        " + ln for ln in self.prologue] + self.lines[body_start:])
+        return self.wrap(body)
+
+    def run_gq(self, gq):
+        """Value-only code of generated quantities (statements `gq`): transformed data and transformed parameters
+        recomputed, then the block; its top-level declarations are the outputs.  -> (struct text, output names)"""
+        program = self.declare_inputs() + self.blocks.get("transformed parameters", []) + list(gq)
+        outputs = [st[1] for st in gq if st[0] == "decl"]
+        for name, base, shape, lo, hi, init, line in outputs:
+            if self.orients.get(name) == "mat":
+                raise StanSubsetError(f"line {line}: matrix outputs of generated quantities are outside the supported "
+                                      f"subset")
+        self.loop_vars = []
+        self.statements(program, emit=True)
+        body = self.lines
+        self.lines = []
+        for v in self.vars.values():         # locals start as NaN, as in Stan
+            if v.kind == "local":
+                self.emit(f"double v_{v.name}{f'[{v.size}]' if v.shape else ''};")
+                self.emit(f"for (int i = 0; i < {v.size}; ++i) v_{v.name}{'[i]' if v.shape else ''} = NAN;"
+                          if v.shape else f"v_{v.name} = NAN;")
+        names, copy = [], []
+        for name, *_ in outputs:
+            v = self.vars[name]
+            copy.append(f"for (int j = 0; j < {v.size}; ++j) out[{len(names)} + j] = v_{name}[j];" if v.shape else
+                        f"out[{len(names)}] = v_{name};")
+            names += [name if not v.shape else f"{name}.{'.'.join(str(i + 1) for i in _unravel(j, v.shape))}"
+                      for j in range(v.size)]
+        if len(names) > self.MAX_GQ:
+            raise StanSubsetError(f"{len(names)} generated quantities; the generated kernels support up to {self.MAX_GQ}")
+        return self.wrap_gq("\n".join(["        " + ln for ln in self.prologue] + self.lines + body), copy, len(names)), names
+
+    def declare_inputs(self):
+        """Data, parameters and the integer constants of transformed data -> the other transformed data statements."""
         # data block
         for name, base, shape, lo, hi, init, line in self.blocks["data"]:
             dims = [self.int_expr(d)[0] for d in shape]
@@ -2048,8 +2265,7 @@ class _Gen:
         if self.cdim > 2 * self.MAX_DIM:
             raise StanSubsetError(f"{self.cdim} constrained parameter values; the generated kernels support up to "
                                   f"{2 * self.MAX_DIM}")
-        # transformed data (integer scalars folded now, everything else computed like a parameter-free local) and
-        # transformed parameters (locals of the density; their declared bounds are validation only) run ahead of the model
+        # transformed data: integer scalars folded now, everything else computed like a parameter-free local
         program = []
         for st in self.blocks.get("transformed data", []):
             if st[0] == "decl" and st[1][1] == "int":
@@ -2061,28 +2277,7 @@ class _Gen:
                     raise StanSubsetError(f"line {line}: {name!r} is not a constant")
             else:
                 program.append(st)
-        program += self.blocks.get("transformed parameters", [])
-        program += self.blocks["model"]
-        self.blocks["model"] = _demote_arrays(self.fuse_vector_densities(program)) if RESTRUCTURE else program
-        # activity analysis (which coordinates can each local depend on): fixpoint over the statement list
-        for _ in range(64):
-            self.changed = False
-            self.loop_vars = []
-            self.statements(self.blocks["model"], emit=False)
-            if not self.changed:
-                break
-        # emission
-        self.loop_vars = []
-        body_start = len(self.lines)
-        for v in self.vars.values():
-            if v.kind == "local":
-                dims = "".join(f"[{n}]" for n in ([v.size] if v.shape else []))
-                self.emit(f"double v_{v.name}{dims}{' = {0.0}' if v.shape else ' = 0.0'};")
-                if v.deps:
-                    self.emit(f"double d_{v.name}{dims}[{max(v.deps) + 1}]{' = {{0.0}}' if v.shape else ' = {0.0}'};")
-        self.statements(self.blocks["model"], emit=True)
-        body = "\n".join(["        " + ln for ln in self.prologue] + self.lines[body_start:])
-        return self.wrap(body)
+        return program
 
     @staticmethod
     def check_vector_data(name, kind, flat, K, line):
@@ -2197,6 +2392,34 @@ struct {self.struct_name} {{
 """
         return text
 
+    def wrap_gq(self, body, copy, G):
+        """The generated-quantities struct (`<model struct>GQ`, text included after the model struct): `copy` moves
+        the outputs to out[0 .. GDIM)."""
+        S = self.struct_name
+        return f"""// GENERATED by smcnuts/model/stan_codegen.py -- do not edit.  Generated quantities of {S} (included after it).
+#pragma once
+#include "stan_rng.cuh"
+struct {S}GQ {{
+    static constexpr int DMAX = {self.dim}, CDIM = {self.cdim}, GDIM = {G};
+    const double* data;
+    SMCB_HD explicit {S}GQ(const smcb::ModelDesc& d) : data(d.data) {{}}
+
+    // out[0 .. GDIM) of the unconstrained row x, drawing from rng; all NaN when a draw's arguments are invalid (Stan
+    // throws) or the block rejects
+    SMCB_HD void generated_quantities(const double (&x)[DMAX], smcb::stan::Rng& rng, double* out) const {{
+        double c[CDIM];
+        {S}::constrain(x, c);
+        bool ok = true;
+{body}
+        if (ok && rng.ok) {{
+            {(chr(10) + '            ').join(copy)}
+        }} else {{
+            for (int k = 0; k < GDIM; ++k) out[k] = NAN;
+        }}
+    }}
+}};
+"""
+
 
 def _flatten(v):
     if isinstance(v, (list, tuple)):
@@ -2233,7 +2456,17 @@ def generate(stan_text, data, struct_name="GenModel"):
     import hashlib
     parser = _Parser(stan_text)
     blocks = parser.program()
+    gq_blocks = dict(blocks)             # run() rewrites the model block in place
     g = _Gen(blocks, data, struct_name, parser.orients, parser.ctypes)
     text = g.run()
-    digest = hashlib.sha256((text + repr(g.blob)).encode()).hexdigest()[:16]
-    return GeneratedSource(struct_name, text, g.dim, g.blob, g.param_names, g.transforms, digest, g.cdim, g.param_unc_names)
+    gq_names, gq_error = [], blocks.get("generated quantities error")
+    gq_text = g.wrap_gq("", [], 0)
+    if gq_error is None and blocks.get("generated quantities"):
+        try:
+            q = _Gen(gq_blocks, data, struct_name, dict(parser.gq_orients), dict(parser.gq_ctypes), value_only=True)
+            gq_text, gq_names = q.run_gq(blocks["generated quantities"])
+        except StanSubsetError as e:
+            gq_error = str(e)
+    digest = hashlib.sha256((text + gq_text + repr(g.blob)).encode()).hexdigest()[:16]
+    return GeneratedSource(struct_name, text, g.dim, g.blob, g.param_names, g.transforms, digest, g.cdim, g.param_unc_names,
+                           gq_text, gq_names, gq_error)

@@ -15,6 +15,7 @@ from tqdm import tqdm
 from . import _cabi, _device as dev
 from .estimate.estimate import Estimate
 from .estimate.estimate_from_tempered import EstimateFromTempered
+from .model.stan_codegen import StanSubsetError
 from .parallel import ShardContext
 from .proposal.nuts import NUTSProposal
 from .proposal.nuts_acc_rej import NUTSProposalWithAccRej
@@ -26,7 +27,7 @@ class SMCSampler:
     def __init__(self, K: int, N: int, target, step_size=None, sample_proposal=None, momentum_proposal=None,
                  lkernel="forwardsLKernel", tempering=False, rng=None, forward_kernel=None, verbose=False,
                  resampling="multinomial", save_history=None, history_budget_bytes=48 << 30, shard=None,
-                 adapt_step_size=0, target_accept=0.8, adapt_mass_matrix=False):
+                 adapt_step_size=0, target_accept=0.8, adapt_mass_matrix=False, generated_quantities=False):
         self.K = K  # Number of iterations
         self.N = N  # Number of particles (global)
         self.target = target
@@ -111,6 +112,17 @@ class SMCSampler:
         self._moved = dev.zeros(self.K + 1)
         self.mean_estimate = np.zeros([self.K + 1, DC])
         self.variance_estimate = np.zeros([self.K + 1, DC])
+
+        # generated quantities of the final particle set (generated models): evaluated once by finish()
+        self.generated_quantities = bool(generated_quantities)
+        if self.generated_quantities:
+            if not hasattr(target, "generated_quantities"):
+                raise TypeError("generated_quantities needs a generated model (GeneratedModel)")
+            if target.source.gq_error is not None:       # fail before the run, not after it
+                raise StanSubsetError(f"generated quantities: {target.source.gq_error}")
+            if target.gq_dim == 0:
+                raise ValueError("generated_quantities=True: the program has no generated quantities")
+        self.gq_draws = self.gq_mean_estimate = self.gq_variance_estimate = None
 
     # History under the reference's names (smc_sampler.py:73-74): host NumPy arrays [K+1, N, D] / [K+1, N], materialised
     # lazily from the device-resident history on first access and cached (this rank's shard when particles are sharded).
@@ -236,6 +248,12 @@ class SMCSampler:
         s.calculate_ess()
         self.update_sampler(self.K, mean_estimate, variance_estimate)
         self.phi[self.K] = s.phi_new
+
+        if self.generated_quantities:
+            # one row per local particle (global index: its stream), paired with the final normalised weights s.wn
+            self.gq_draws = self.target.generated_quantities(s.x, seed=self.seed, counter=0, particle0=s.offset)
+            gq_mean, gq_var = Estimate(self.target, shard=self.shard).return_estimate_unconstrained(self.gq_draws, s.wn)
+            self.gq_mean_estimate, self.gq_variance_estimate = gq_mean.cpu().numpy(), gq_var.cpu().numpy()
 
         torch.cuda.synchronize()
         self.leapfrogs = self.shard.all_reduce_sum_(self._lf.clone()).cpu().numpy()
