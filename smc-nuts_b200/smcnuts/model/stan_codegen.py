@@ -46,7 +46,21 @@ Supported subset (anything else raises StanSubsetError with the offending line):
   neg_binomial_2_log mass functions --
   scalar or vectorised over container arguments and container-valued argument expressions;  dirichlet (alpha data or
   parameters), categorical (an int or int array outcome) and multinomial (an int array) of a vector argument, the integer
-  outcomes being data known at generation time (tabulated into counts).
+  outcomes being data known at generation time (tabulated into counts);
+  matrices: cholesky_decompose(A) (symmetric within 1e-8 and positive definite, else the density is -inf), add_diag(A, d)
+  (d real or vector), gp_exp_quad_cov(x, alpha, rho) (x array[] real or array[] vector), multi_normal_lpdf(y | mu, Sigma)
+  and multi_normal_cholesky_lpdf(y | mu, L) (y and mu vectors or arrays of vectors; only the lower triangle of L is read,
+  a diagonal entry <= 0 or not finite gives -inf; `~` drops -K/2 log 2 pi, and -sum log L_ii when the matrix depends on no
+  parameter) -- lowered onto element loops of the scalar subset (`_Gen.mvn_terms`, `_Gen.cholesky_in_place`), the factor
+  computed in place in the assigned matrix, loops with literal bounds kept rolled.  A covariance of multi_normal that is a
+  data variable, and `matrix[K, K] L = cholesky_decompose(S);` in transformed data with S a data variable, are factored
+  when the model is generated (numpy; not symmetric positive definite -> StanSubsetError with the line): an evaluation
+  then only solves, O(K^2).
+  Per-thread budget: the matrix locals of the density, values and tangents (8 bytes x entries x (1 + tangents an entry,
+  the highest coordinate the matrix depends on + 1)), take at most _Gen.MAX_MATRIX_BYTES = 32 KiB; a program past it is
+  refused with the line of the matrix that crosses it.  Local memory is reserved for every thread that can be resident
+  (148 SMs x 2048 on a B200), so 32 KiB is about 10 GB of the device: the plug-in's NUTS kernel has a 34 KB stack frame
+  at the budget (a 32-observation GP with 3 hyperparameters, profiles/gp_time.log).
 
 Generated quantities (a separate output: `constrain()`, `param_names` and the density code do not change)
   a second struct `<struct_name>GQ` (GeneratedSource.gq_text) with generated_quantities(x, rng, out): value-only code
@@ -56,7 +70,9 @@ Generated quantities (a separate output: `constrain()`, `param_names` and the de
   by value (`normal_lpdf(y[n] | mu[n], sigma)`), plus the _rng functions of csrc/stan_rng.cuh: normal, std_normal,
   student_t, cauchy, double_exponential, logistic, lognormal, exponential, gamma, inv_gamma, beta, uniform, bernoulli,
   bernoulli_logit, binomial, poisson, poisson_log, neg_binomial_2 (scalar, or vectorised into arrays) and categorical (of a
-  vector).  `target +=`, `~`, phi and redeclared names are refused there, _rng calls everywhere else; G is at most
+  vector), and multi_normal_rng(mu, Sigma) / multi_normal_cholesky_rng(mu, L) (a vector mean; K standard normals drawn
+  in coordinate order, then mu + L z; into a vector or an element of an array of vectors; data covariances are factored
+  per evaluation here).  `target +=`, `~`, phi and redeclared names are refused there, _rng calls everywhere else; G is at most
   MAX_GQ (one row of a particle block fits in shared memory).  A block outside this subset does
   not stop the model: its StanSubsetError text (with the line) is kept in GeneratedSource.gq_error and raised when gq
   values are requested.
@@ -622,6 +638,20 @@ _DENSITIES = {
 }
 # densities of a whole vector argument (simplex-valued or counts), lowered by _Gen.vector_density
 _VECTOR_DENSITIES = ("dirichlet", "categorical", "multinomial")
+# multivariate normal densities of vectors (or arrays of them) under a covariance or its Cholesky factor (_Gen.mvn_terms)
+_MVN_DENSITIES = ("multi_normal", "multi_normal_cholesky")
+_MVN_RNGS = ("multi_normal_rng", "multi_normal_cholesky_rng")
+# matrix functions lowered onto element loops; the loops with literal bounds of a statement that uses one stay rolled
+# (`#pragma unroll 1`): fully unrolled, the O(N^3) nests of a factorisation multiply nvcc time, code size and spills
+_MATRIX_FUNCS = ("cholesky_decompose", "add_diag", "gp_exp_quad_cov", "multi_normal_lpdf",
+                 "multi_normal_cholesky_lpdf") + _MVN_RNGS
+_DBL_MAX = 1.7976931348623157e308
+
+
+def _calls_any(e, names):
+    found = []
+    _walk_exprs(e, lambda x: found.append(x) if x[0] == "call" and x[1] in names else None)
+    return bool(found)
 
 
 def _sum_exprs(terms, line):
@@ -866,12 +896,20 @@ class GeneratedSource:
 class _Gen:
     MAX_DIM = 64
     MAX_GQ = 24576          # outputs of generated quantities: a row of a particle block fits in shared memory
+    # matrix locals of one thread, values and tangents together (module docstring): every thread that can be resident
+    # (148 SMs x 2048 on a B200) gets a stack frame of at least this much local memory, about 10 GB at 32 KiB
+    MAX_MATRIX_BYTES = 32768
 
     def __init__(self, blocks, data, struct_name, orients=None, ctypes=None, value_only=False):
         self.blocks, self.struct_name = blocks, struct_name
         self.value_only = value_only    # generated quantities: values only (no sensitivities, no A / B split), _rng calls
         self.orients = orients or {}
         self.ctypes = ctypes or {}
+        self.rolled = set()     # loop variables of matrix-function lowerings: emitted with `#pragma unroll 1`
+        self.rolling = False    # while a statement that uses a matrix function is lowered: its fresh loops are rolled
+        self.materialized = {}  # id(matrix-valued call) -> the local it is computed into (one statement's lowering)
+        self.folded = {}        # data covariance name -> name of its Cholesky factor, computed at generation time
+        self.decl_lines = {}    # local name -> line of its declaration
         self.lowered = {}       # id(statement) -> its scalar-subset replacement (list of statements) or None
         self.rng_stmts = {}     # id(statement) -> the statement with its draws ahead of it, or None (value-only mode)
         self.scopes = [set()]   # value-only mode: names declared in each enclosing scope (Stan refuses redeclarations)
@@ -965,6 +1003,11 @@ class _Gen:
         k = e[0]
         if k == "num":
             return _const(e[1])
+        if k == "ideq":          # 1.0 where two integer expressions are equal, else 0.0 (the diagonal of add_diag)
+            (va, ca), (vb, cb) = self.int_expr(e[1]), self.int_expr(e[2])
+            if va is not None and vb is not None:
+                return _const(1.0 if va == vb else 0.0)
+            return Node("ivar", name=f"({ca} == {cb})")
         if k == "neg":
             return _un("neg", self.real(e[1]))
         if k == "bin":
@@ -1102,7 +1145,7 @@ class _Gen:
     def shape(self, e):
         """-> (dims tuple, orientation of a 1-d result: "col" | "row" | None, or "mat")"""
         k = e[0]
-        if k == "num":
+        if k == "num" or k == "ideq":
             return (), None
         if k == "var" or k == "idx":
             base, idx = (e, []) if k == "var" else (e[1], e[2])
@@ -1158,6 +1201,8 @@ class _Gen:
                 return (n,), {"rep_vector": "col", "rep_row_vector": "row", "rep_array": None}[name]
             if name == "categorical_rng":
                 return (), None
+            if name in ("cholesky_decompose", "add_diag", "gp_exp_quad_cov") + _MVN_RNGS:
+                return self.matrix_call_shape(name, args, e[3])
             shapes = [self.shape(a) for a in args]
             big = [sh for sh in shapes if sh[0]]
             if big and any(sh[0] != big[0][0] for sh in big):
@@ -1169,7 +1214,10 @@ class _Gen:
 
     def fresh_name(self, prefix):
         self.fresh += 1
-        return f"{prefix}__{self.fresh}"       # Stan identifiers cannot end in two underscores: no collisions
+        name = f"{prefix}__{self.fresh}"       # Stan identifiers cannot end in two underscores: no collisions
+        if self.rolling:
+            self.rolled.add(name)
+        return name
 
     def reduce(self, n, term_of, pre, line):
         """acc = sum over k = 1..n of term_of(k), emitted as scalar-subset statements appended to `pre` -> the accumulator"""
@@ -1191,7 +1239,7 @@ class _Gen:
             raise StanSubsetError(f"line {line}: a container of {len(dims)} dimension(s) is used where {len(ix)} are expected")
         if not dims and self.outer_pre is not None:
             pre = self.outer_pre
-        if k == "num":
+        if k == "num" or k == "ideq":
             return e
         if k == "var":
             return ("idx", e, list(ix)) if ix else e
@@ -1217,6 +1265,24 @@ class _Gen:
             name, args, cl = e[1], e[2], e[3]
             if name in self._REPS and len(args) == 2:
                 return self.lower(args[0], [], pre, cl)
+            if name == "add_diag":
+                i, j = ix
+                d = args[1]
+                dv = self.lower(d, [i] if self.shape(d)[0] else [], pre, cl)
+                return ("bin", "+", self.lower(args[0], ix, pre, cl), ("bin", "*", ("ideq", i, j), dv))
+            if name == "gp_exp_quad_cov":
+                x, alpha, rho = args
+                xd = self.shape(x)[0]
+                if len(xd) == 1:
+                    d2 = ("call", "square", [("bin", "-", self.lower(x, [ix[0]], pre, cl), self.lower(x, [ix[1]], pre, cl))], cl)
+                else:
+                    d2 = self.reduce(xd[1], lambda kk, p2: ("call", "square", [("bin", "-", self.lower(x, [ix[0], kk], p2, cl),
+                                                                                  self.lower(x, [ix[1], kk], p2, cl))], cl), pre, cl)
+                scale = ("bin", "/", ("num", -0.5, False), ("call", "square", [self.lower(rho, [], pre, cl)], cl))
+                return ("bin", "*", ("call", "square", [self.lower(alpha, [], pre, cl)], cl),
+                        ("call", "exp", [("bin", "*", d2, scale)], cl))
+            if name == "cholesky_decompose" or name in _MVN_RNGS:
+                return ("idx", self.materialize(e, pre, cl), list(ix))
             if name in self._REDUCTIONS:
                 shapes = [self.shape(a)[0] for a in args]
                 if len(args) != (2 if name == "dot_product" else 1) or any(len(d) != 1 for d in shapes) or len(set(shapes)) != 1:
@@ -1248,6 +1314,8 @@ class _Gen:
             m = re.fullmatch(r"(\w+?)_(lpdf|lpmf|log)", name)
             if m and m.group(1) in _VECTOR_DENSITIES:
                 return _sum_exprs(self.vector_density(m.group(1), args, pre, cl), cl)
+            if m and m.group(1) in _MVN_DENSITIES:
+                return _sum_exprs(self.mvn_terms(m.group(1), args, pre, cl), cl)
             if m and m.group(1) in _DENSITIES:
                 shapes = [self.shape(a)[0] for a in args]
                 big = [d for d in shapes if d]
@@ -1342,6 +1410,246 @@ class _Gen:
         norm = math.lgamma(sum(ys) + 1.0) - math.fsum(math.lgamma(z + 1.0) for z in ys)
         return [("num", norm, False), weighted_logs(theta, ys)]
 
+    # ---- matrices: cholesky_decompose, add_diag, gp_exp_quad_cov, multi_normal(_cholesky) densities and draws -----------
+    # All of them are lowered onto rolled element loops of the scalar subset, so that the tangents follow the existing
+    # activity analysis (only the coordinates a matrix can depend on).  The factor is computed in place in the assigned
+    # matrix; a covariance that is a data variable is factored when the model is generated (fold_cholesky).
+    def square_dim(self, e, what, line):
+        dims, orient = self.shape(e)
+        if orient != "mat" or dims[0] != dims[1]:
+            raise StanSubsetError(f"line {line}: {what} takes a square matrix (found a container of size {list(dims)})")
+        return dims[0]
+
+    def matrix_call_shape(self, name, args, line):
+        arity = {"cholesky_decompose": 1, "add_diag": 2, "gp_exp_quad_cov": 3}.get(name, 2)
+        if len(args) != arity:
+            raise StanSubsetError(f"line {line}: {name} takes {arity} argument(s)")
+        if name == "gp_exp_quad_cov":
+            (dx, ox), ds = self.shape(args[0]), [self.shape(a)[0] for a in args[1:]]
+            if ox is not None or len(dx) not in (1, 2) or any(ds):
+                raise StanSubsetError(f"line {line}: gp_exp_quad_cov(x, alpha, rho) takes x as array[] real or array[] vector "
+                                      f"and real alpha and rho")
+            return (dx[0], dx[0]), "mat"
+        if name in _MVN_RNGS:
+            n = self.square_dim(args[1], name, line)
+            dm, om = self.shape(args[0])
+            if dm != (n,) or om not in ("col", "row"):
+                raise StanSubsetError(f"line {line}: {name} takes a vector mean of size {n} (found a container of size "
+                                      f"{list(dm)})")
+            return (n,), "col"
+        n = self.square_dim(args[0], name, line)
+        if name == "add_diag" and self.shape(args[1])[0] not in ((), (n,)):
+            raise StanSubsetError(f"line {line}: add_diag adds a real or a vector of size {n}")
+        return (n, n), "mat"
+
+    def loop(self, lo, hi, body_of, line):
+        """`for (v in lo:hi) { body_of(v) }` with a fresh, rolled loop variable"""
+        v = self.fresh_name("i")
+        self.rolled.add(v)
+        return ("for", v, lo, hi, [("block", body_of(("var", v, line)), line)], line)
+
+    def local(self, dims, orient, line, init=None, prefix="t"):
+        """a fresh local (declared now, so that the expressions built next can use it) and its declaration"""
+        name = self.fresh_name(prefix)
+        if orient:
+            self.orients[name] = orient
+        self.vars[name] = _Var(name, "local", list(dims), "real", orient=orient)
+        return ("var", name, line), ("decl", (name, "real", [("num", float(d), True) for d in dims], None, None, init, line),
+                                     line)
+
+    def materialize(self, e, pre, line):
+        """a matrix- or vector-valued call computed once, ahead of the statement, into a fresh local -> its name"""
+        if id(e) not in self.materialized:
+            dims, orient = self.shape(e)
+            tmp, decl = self.local(dims, orient, line, prefix="m")
+            out = self.outer_pre if self.outer_pre is not None else pre
+            out.append(decl)
+            out += self._lower_stmt_inner(("assign", tmp, "=", e, line), [])
+            self.materialized[id(e)] = (e, tmp)
+        return self.materialized[id(e)][1]
+
+    def matrix_assign(self, lhs, rhs, line):
+        """statements that assign cholesky_decompose(A) or a multi_normal(_cholesky)_rng draw to the whole container lhs"""
+        name, args = rhs[1], rhs[2]
+        one = ("num", 1.0, True)
+        if name == "cholesky_decompose":
+            n = self.square_dim(args[0], name, line)
+            copy = self._lower_stmt_inner(("assign", lhs, "=", args[0], line), [])
+            return copy + self.cholesky_in_place(lambda i, j: self.lower(lhs, [i, j], [], line), n, line)
+        if not self.value_only:
+            raise StanSubsetError(f"line {line}: {name}: _rng functions are only allowed in generated quantities")
+        mu, S = args
+        (n,), _ = self.shape(rhs)
+        if name == "multi_normal_rng":
+            S = self.materialize(("call", "cholesky_decompose", [S], line), [], line)
+        elif S[0] not in ("var", "idx"):
+            S = self.materialize(S, [], line)
+        z, decl = self.local([n], "col", line, prefix="z")
+        t = self.fresh_name("t")
+
+        def mu_at(i, pre):
+            return self.lower(mu, [i], pre, line)
+
+        def finite(i):
+            pre = []
+            m = mu_at(i, pre)
+            return pre + [("if", ("lnot", ("cmp", "<=", ("call", "fabs", [m], line), ("num", _DBL_MAX, False))),
+                           ("reject", line), None, line)]
+
+        def row(i):
+            pre = []
+            m = mu_at(i, pre)
+            return pre + [("decl", (t, "real", [], None, None, m, line), line),
+                          self.loop(one, i, lambda j: [("assign", ("var", t, line), "+=",
+                                                        ("bin", "*", self.lower(S, [i, j], [], line), ("idx", z, [j])), line)],
+                                    line),
+                          ("assign", self.lower(lhs, [i], [], line), "=", ("var", t, line), line)]
+        nn = ("num", float(n), True)
+        # K standard normals in coordinate order, then mu + L z (Stan checks that mu is finite; the factor of Sigma, that
+        # Sigma is symmetric positive definite)
+        return [decl, self.loop(one, nn, lambda i: [("assign", ("idx", z, [i]), "=", ("call", "std_normal_rng", [], line),
+                                                     line)], line),
+                self.loop(one, nn, finite, line), self.loop(one, nn, row, line)]
+
+    def cholesky_in_place(self, E, n, line):
+        """Statements that replace the n x n matrix of elements E(i, j) (index expressions) by its lower Cholesky factor,
+        column by column (each column reads the input's lower triangle and the finished columns only); then zero the
+        upper triangle.  As Stan Math: the input is symmetric within 1e-8 (which NaN and infinite entries fail) and
+        positive definite, or the density is -inf (reject)."""
+        one, nn = ("num", 1.0, True), ("num", float(n), True)
+        rej = ("reject", line)
+
+        def minus1(v):
+            return ("bin", "-", v, one)
+
+        def not_le(a, b):
+            return ("lnot", ("cmp", "<=", a, ("num", b, False)))
+        check = self.loop(one, nn, lambda i: [self.loop(one, i, lambda j: [
+            ("if", not_le(("call", "fabs", [("bin", "-", E(i, j), E(j, i))], line), 1e-8), rej, None, line)], line)], line)
+
+        def column(j):
+            s, t = self.fresh_name("s"), self.fresh_name("t")
+
+            def row(i):
+                return [("decl", (t, "real", [], None, None, E(i, j), line), line),
+                        self.loop(one, minus1(j), lambda k: [("assign", ("var", t, line), "-=", ("bin", "*", E(i, k), E(j, k)),
+                                                              line)], line),
+                        ("assign", E(i, j), "=", ("bin", "/", ("var", t, line), E(j, j)), line)]
+            return [("decl", (s, "real", [], None, None, E(j, j), line), line),
+                    self.loop(one, minus1(j), lambda k: [("assign", ("var", s, line), "-=", ("call", "square", [E(j, k)], line),
+                                                          line)], line),
+                    ("if", ("lnot", ("cmp", ">", ("var", s, line), ("num", 0.0, False))), rej, None, line),
+                    ("assign", E(j, j), "=", ("call", "sqrt", [("var", s, line)], line), line),
+                    self.loop(("bin", "+", j, one), nn, row, line)]
+        upper = self.loop(one, nn, lambda i: [self.loop(("bin", "+", i, one), nn, lambda j: [
+            ("assign", E(i, j), "=", ("num", 0.0, True), line)], line)], line)
+        return [check, self.loop(one, nn, column, line), upper]
+
+    def cholesky_of_data(self, name, line):
+        """Stan's cholesky_decompose of the data matrix `name`, now: the factor's values (row-major); a matrix that is not
+        symmetric (within 1e-8) positive definite with finite entries is refused"""
+        import numpy as np
+        v = self.vars[name]
+        n = v.shape[-1]
+        a = np.array(v.value, dtype=np.float64).reshape(n, n)
+        fac = None
+        if np.all(np.isfinite(a)) and np.all(np.abs(a - a.T) <= 1e-8):
+            try:
+                fac = np.linalg.cholesky(a)
+            except np.linalg.LinAlgError:
+                pass
+        if fac is None or not np.all(np.diag(fac) > 0.0):
+            raise StanSubsetError(f"line {line}: data {name!r} is not a symmetric positive definite matrix")
+        return [float(z) for z in fac.ravel()]
+
+    def data_matrix(self, name, n, values):
+        self.vars[name] = _Var(name, "data", [n, n], "real", offset=len(self.blob), value=values, orient="mat")
+        self.orients[name] = "mat"
+        self.blob += values
+
+    def fold_cholesky(self, name, line):
+        """the Cholesky factor of data covariance `name`, computed once at generation time into the data blob"""
+        if name not in self.folded:
+            values = self.cholesky_of_data(name, line)
+            self.folded[name] = self.fresh_name(f"{name}_chol")
+            self.data_matrix(self.folded[name], self.vars[name].shape[-1], values)
+        return self.folded[name]
+
+    def mvn_terms(self, dist, args, pre, line):
+        """multi_normal(_cholesky)_lpdf(y | mu, S) -> its terms [-M K/2 log 2 pi, -M sum_i log L_ii, -1/2 sum_n |z_n|^2]
+        with z_n = L^-1 (y_n - mu_n) by forward substitution (M vectors y_n / mu_n); the statements that compute the
+        factor, log-determinant and quadratic form go to `pre`.  Under `~` the first term is always dropped and the second
+        one when L depends on no parameter (ptarget)."""
+        if len(args) != 3:
+            raise StanSubsetError(f"line {line}: {dist} takes 3 arguments")
+        y, mu, S = args
+        K = self.square_dim(S, dist, line)
+
+        def count(e, what):      # -> number of vectors of an array (None for one vector)
+            d, o = self.shape(e)
+            if len(d) == 1 and o in ("col", "row"):
+                m, k = None, d[0]
+            elif len(d) == 2 and o is None:
+                m, k = d
+            else:
+                raise StanSubsetError(f"line {line}: {dist}: {what} must be a vector or an array of vectors")
+            if k != K:
+                raise StanSubsetError(f"line {line}: {dist}: {what} has {k} elements, the matrix is {K} x {K}")
+            return m
+        my, mm = count(y, "the outcome"), count(mu, "the location")
+        if my is not None and mm is not None and my != mm:
+            raise StanSubsetError(f"line {line}: {dist}: arrays of {my} outcomes and {mm} locations")
+        M = my or mm or 1
+        one, kk = ("num", 1.0, True), ("num", float(K), True)
+        checked = False
+        if dist == "multi_normal":
+            if S[0] == "var" and self.vars[S[1]].kind == "data" and not self.value_only:
+                S = ("var", self.fold_cholesky(S[1], line), line)
+            else:
+                S, checked = self.materialize(("call", "cholesky_decompose", [S], line), pre, line), True
+        elif S[0] not in ("var", "idx"):
+            S = self.materialize(S, pre, line)
+
+        def E(i, j):
+            return self.lower(S, [i, j], [], line)
+        if S[0] == "var" and self.vars[S[1]].kind == "data":          # log-determinant of a data factor: folded now
+            diag = [self.vars[S[1]].value[i * K + i] for i in range(K)]
+            if all(0.0 < d < math.inf for d in diag):
+                ld = ("num", math.fsum(math.log(d) for d in diag), False)
+            else:
+                pre.append(("reject", line))
+                ld = ("num", 0.0, False)
+        else:
+            ld, decl = self.local([], None, line, ("num", 0.0, True), prefix="ld")
+            pre.append(decl)
+            dg = lambda i: E(i, i)           # noqa: E731
+
+            def diag(i):
+                bad = ("lor", ("lnot", ("cmp", ">", dg(i), ("num", 0.0, False))),
+                       ("lnot", ("cmp", "<=", dg(i), ("num", _DBL_MAX, False))))
+                return ([] if checked else [("if", bad, ("reject", line), None, line)]) + \
+                    [("assign", ld, "+=", ("call", "log", [dg(i)], line), line)]
+            pre.append(self.loop(one, kk, diag, line))
+        q, qdecl = self.local([], None, line, ("num", 0.0, True), prefix="q")
+        z, zdecl = self.local([K], "col", line, prefix="z")
+        t = self.fresh_name("t")
+
+        def solve(n):
+            def row(i):
+                inner = []
+                yi = self.lower(y, [i] if my is None else [n, i], inner, line)
+                mi = self.lower(mu, [i] if mm is None else [n, i], inner, line)
+                return inner + [("decl", (t, "real", [], None, None, ("bin", "-", yi, mi), line), line),
+                                self.loop(one, ("bin", "-", i, one), lambda j: [
+                                    ("assign", ("var", t, line), "-=", ("bin", "*", E(i, j), ("idx", z, [j])), line)], line),
+                                ("assign", ("idx", z, [i]), "=", ("bin", "/", ("var", t, line), E(i, i)), line),
+                                ("assign", q, "+=", ("call", "square", [("idx", z, [i])], line), line)]
+            return [self.loop(one, kk, row, line)]
+        pre += [qdecl, zdecl]
+        pre += [self.loop(one, ("num", float(M), True), solve, line)] if M > 1 else solve(None)
+        return [("num", -0.5 * M * K * _LOG_2PI, False), ("neg", ("bin", "*", ("num", float(M), False), ld)),
+                ("bin", "*", ("num", -0.5, False), q)]
+
     def is_plain(self, e):
         """Expressions the scalar machinery takes as they are: scalars without container operations inside, and whole
         one-dimensional variables (the vectorised density arguments of target_terms)."""
@@ -1370,10 +1678,13 @@ class _Gen:
 
     def _lower_stmt(self, s):
         self.outer_pre = []
+        self.rolling = (s[0] == "tilde" and s[2] in _MVN_DENSITIES) or _calls_any(s, _MATRIX_FUNCS)
+        self.materialized = {}
         try:
             out = self._lower_stmt_inner(s, self.outer_pre)
         finally:
             self.outer_pre = None
+            self.rolling = False
         return out
 
     @staticmethod
@@ -1401,6 +1712,8 @@ class _Gen:
                 tempered, dist, args = False, s[2], [s[1]] + s[3]
                 if dist in _VECTOR_DENSITIES:       # propto: a term that depends on no parameter is dropped when emitted
                     return pre + [("ptarget", t, line) for t in self.vector_density(dist, args, pre, line)]
+                if dist in _MVN_DENSITIES:
+                    return pre + [("ptarget", t, line) for t in self.mvn_terms(dist, args, pre, line)]
 
             def rebuild(a):
                 if kind == "tilde":
@@ -1433,6 +1746,10 @@ class _Gen:
             _, lhs, op, rhs, _ = s
             ldims, _ = self.shape(lhs)
             rdims, _ = self.shape(rhs)
+            if op == "=" and rhs[0] == "call" and rhs[1] in ("cholesky_decompose",) + _MVN_RNGS:
+                if rdims != ldims:
+                    raise StanSubsetError(f"line {line}: assignment of a container of size {rdims} to one of size {ldims}")
+                return pre + self.matrix_assign(lhs, rhs, line)
             if not ldims:
                 r2 = self.lower(rhs, [], pre, line)
                 return None if (r2 == rhs and not pre) else pre + [("assign", lhs, op, r2, line)]
@@ -2082,6 +2399,7 @@ class _Gen:
                     if any(name in sc for sc in self.scopes):
                         raise StanSubsetError(f"line {line}: {name!r} is already declared")
                     self.scopes[-1].add(name)
+                self.decl_lines.setdefault(name, line)
                 dims = []
                 for d in shape:
                     dv, _ = self.int_expr(d)
@@ -2101,7 +2419,10 @@ class _Gen:
                 cname = f"{var}_{len(self.loop_vars)}"
                 if emit:
                     trip = (hiv - lov + 1) if (lov is not None and hiv is not None) else None
-                    if trip is not None and trip <= 16:
+                    if var in self.rolled:          # literal bounds: never fully unrolled; others: nvcc's default
+                        if trip is not None:
+                            self.emit("#pragma unroll 1")
+                    elif trip is not None and trip <= 16:
                         self.emit("#pragma unroll")
                     self.emit(f"for (int {cname} = {loc}; {cname} <= {hic}; ++{cname}) {{")
                     self.indent += 1
@@ -2153,6 +2474,7 @@ class _Gen:
             self.statements(self.blocks["model"], emit=False)
             if not self.changed:
                 break
+        self.check_matrix_budget()
         # emission
         self.loop_vars = []
         body_start = len(self.lines)
@@ -2177,6 +2499,7 @@ class _Gen:
                                       f"subset")
         self.loop_vars = []
         self.statements(program, emit=True)
+        self.check_matrix_budget()
         body = self.lines
         self.lines = []
         for v in self.vars.values():         # locals start as NaN, as in Stan
@@ -2194,6 +2517,43 @@ class _Gen:
         if len(names) > self.MAX_GQ:
             raise StanSubsetError(f"{len(names)} generated quantities; the generated kernels support up to {self.MAX_GQ}")
         return self.wrap_gq("\n".join(["        " + ln for ln in self.prologue] + self.lines + body), copy, len(names)), names
+
+    def check_matrix_budget(self):
+        """Refuses a program whose matrix locals, values and tangents, take more than MAX_MATRIX_BYTES a thread (named
+        with the declaration that crosses the budget)."""
+        total = 0
+        for v in self.vars.values():
+            if v.kind == "local" and v.orient == "mat":
+                nd = max(v.deps) + 1 if v.deps else 0
+                total += 8 * v.size * (1 + nd)
+                if total > self.MAX_MATRIX_BYTES:
+                    raise StanSubsetError(
+                        f"line {self.decl_lines.get(v.name, '?')}: matrix locals take {total} bytes a thread up to "
+                        f"{v.name.split('__')[0]!r} ({' x '.join(map(str, v.shape))}, {1 + nd} double(s) an entry with "
+                        f"its tangents); the generated kernels allow up to {self.MAX_MATRIX_BYTES}")
+
+    def fold_data_cholesky(self, st):
+        """`matrix[K, K] L = cholesky_decompose(S);` in transformed data, with S a data matrix and L assigned nowhere
+        else: L becomes data, factored now (True), instead of a local factored in every evaluation"""
+        if st[0] != "decl" or self.value_only:
+            return False
+        name, _, shape, _, _, init, line = st[1]
+        if not (init is not None and init[0] == "call" and init[1] == "cholesky_decompose" and len(init[2]) == 1
+                and init[2][0][0] == "var" and self.orients.get(name) == "mat"):
+            return False
+        src = self.vars.get(init[2][0][1])
+        if src is None or src.kind != "data" or src.orient != "mat":
+            return False
+        others = [s for blk in ("transformed data", "transformed parameters", "model") for s in self.blocks.get(blk, [])
+                  if s is not st]
+        if name in _assigned_names(others, set()):
+            return False
+        n = self.square_dim(init[2][0], "cholesky_decompose", line)
+        if [self.int_expr(d)[0] for d in shape] != [n, n]:
+            raise StanSubsetError(f"line {line}: assignment of a {n} x {n} factor to {name!r} of size "
+                                  f"{[self.int_expr(d)[0] for d in shape]}")
+        self.data_matrix(name, n, self.cholesky_of_data(src.name, line))
+        return True
 
     def declare_inputs(self):
         """Data, parameters and the integer constants of transformed data -> the other transformed data statements."""
@@ -2275,7 +2635,7 @@ class _Gen:
                 self.vars[name] = _Var(name, "data", [], "int", value=self.int_expr(init)[0])
                 if self.vars[name].value is None:
                     raise StanSubsetError(f"line {line}: {name!r} is not a constant")
-            else:
+            elif not self.fold_data_cholesky(st):
                 program.append(st)
         return program
 
