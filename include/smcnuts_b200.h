@@ -227,6 +227,11 @@ int smcb_gather_rows(const double* x, const int64_t* idx, long long M, int D, do
 
 /* out[i][d] = x[i][d] * scale[d] (inverse = 0) or x[i][d] / scale[d] (inverse = 1); scale is a device array of D doubles */
 int smcb_scale_rows(const double* x, long long N, int D, const double* scale, int inverse, double* out, void* stream);
+/* out[i][d] = accepted[i] ? z[i][d] * scale[d] : x[i][d] -- the way back to x-space after a diagonal-metric transition with
+ * the MH epilogue: a rejected particle keeps its x row exactly (z * scale with z = x / scale can differ from x in the last
+ * bit).  out may be z (in place), not x. */
+int smcb_scale_rows_accepted(const double* z, const int* accepted, const double* x, long long N, int D, const double* scale,
+                             double* out, void* stream);
 
 /* ---- estimators (estimate.py:79-95 with constrain fused, bridgestan.py:93-120) */
 /* out[d] = sum_i wn_i * (c(x_i)_d - center_d)^power ; center may be NULL (0), power in {1, 2} */

@@ -88,6 +88,14 @@ SMCB_HD int ctz32(uint32_t v) {
     return __builtin_ctz(v);
 #endif
 }
+// a * b rounded on its own: never contracted into an FMA with a neighbouring addition
+SMCB_HD double mul_rn(double a, double b) {
+#if defined(__CUDA_ARCH__)
+    return __dmul_rn(a, b);
+#else
+    return a * b;
+#endif
+}
 SMCB_HD double neg_inf() {
 #if defined(__CUDA_ARCH__)
     return __longlong_as_double(0xfff0000000000000ULL);

@@ -552,7 +552,7 @@ struct ScaledModel : M {
     SMCB_HD explicit ScaledModel(const ModelDesc& d, const double* staged) : M(d, staged), scale(d.scale), d_(d.dim) {}
     SMCB_HD void eval(const double (&z)[M::NLOC], double phi, double& A, double& B, double (&g)[M::NLOC]) const {
         double x[M::NLOC], s[M::NLOC];
-#if defined(SMCB_WARP_CODE) && defined(__CUDA_ARCH__)
+#if defined(SMCB_WARP_CODE)   // the device, and the warp emulator of tests/hostsim: lane `sub` of a group
         const int sub = (M::GROUP == 1) ? 0 : (int)(threadIdx.x % M::GROUP);
 #else
         const int sub = 0;
@@ -562,11 +562,16 @@ struct ScaledModel : M {
         for (int i = 0; i < (M::STATIC_NL ? M::STATIC_NL : n); ++i) {
             const int c = (M::GROUP == 1) ? i : sub + M::GROUP * i;
             s[i] = (c < d_) ? SMCB_LDG(&scale[c]) : 1.0;
-            x[i] = z[i] * s[i];
+            x[i] = mul_rn(z[i], s[i]);
         }
+        // mul_rn: with plain products nvcc is free to fuse them with the model's arithmetic, and it compiles the
+        // wrapped model differently from the unwrapped one (arma: 178 DMUL in the kernel against 166 with mul_rn, same
+        // DFMA count, a different schedule; the differing instruction was not traced).  MEASURED on B200: scale = ones
+        // then left x_new 1 ulp away from the identity-metric kernel in 122 of 2061 one-lane PRMwCD rows; with mul_rn the
+        // two agree bit for bit at every dispatch tests/test_metric_kernels.py runs.
         M::eval(x, phi, A, B, g);
 #pragma unroll
-        for (int i = 0; i < (M::STATIC_NL ? M::STATIC_NL : n); ++i) g[i] *= s[i];
+        for (int i = 0; i < (M::STATIC_NL ? M::STATIC_NL : n); ++i) g[i] = mul_rn(g[i], s[i]);
     }
 };
 

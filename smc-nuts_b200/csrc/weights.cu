@@ -726,6 +726,17 @@ __global__ void scale_rows_kernel(const double* __restrict__ x, long long n_elem
     }
 }
 
+// out[i][d] = accepted[i] ? z[i][d] * scale[d] : x[i][d]: back to x-space after a diagonal-metric transition with the MH
+// epilogue, where a rejected particle must keep its x row (the kernel returned z = x / scale for it, and z * scale need not
+// round back to x).  out may alias z.
+__global__ void scale_rows_accepted_kernel(const double* z, const int* __restrict__ accepted, const double* __restrict__ x,
+                                           long long n_elem, int D, const double* __restrict__ scale, double* out) {
+    for (long long e = blockIdx.x * (long long)blockDim.x + threadIdx.x; e < n_elem; e += (long long)gridDim.x * blockDim.x) {
+        const int d = (int)(e % D);
+        out[e] = accepted[e / D] ? z[e] * scale[d] : x[e];
+    }
+}
+
 // ------------------------------------------------------------------------------------------ FP64 probe
 __global__ void probe_fp64_kernel(int iters, double* sink) {
     double a0 = threadIdx.x * 1e-9, a1 = a0 + 1, a2 = a0 + 2, a3 = a0 + 3, a4 = a0 + 4, a5 = a0 + 5, a6 = a0 + 6, a7 = a0 + 7;
@@ -1028,6 +1039,15 @@ int smcb_scale_rows(const double* x, long long N, int D, const double* scale, in
     if (N == 0) return 0;
     scale_rows_kernel<<<stride_grid(N * D, 256, 8), 256, 0, (cudaStream_t)stream>>>(x, N * D, D, scale, inverse, out);
     return check_launch("scale_rows_kernel");
+}
+
+int smcb_scale_rows_accepted(const double* z, const int* accepted, const double* x, long long N, int D, const double* scale,
+                             double* out, void* stream) {
+    SMCB_REQUIRE(z && accepted && x && scale && out && N >= 0 && D >= 1 && out != x, "bad argument");
+    if (N == 0) return 0;
+    scale_rows_accepted_kernel<<<stride_grid(N * D, 256, 8), 256, 0, (cudaStream_t)stream>>>(z, accepted, x, N * D, D, scale,
+                                                                                             out);
+    return check_launch("scale_rows_accepted_kernel");
 }
 
 int smcb_weighted_moments12(const double* x, const double* wn, long long N, int D, int constrain, const double* center,

@@ -85,6 +85,7 @@ _SIGS = {
     "smcb_sum_int32": [_vp, _ll, _vp, _vp, _vp],
     "smcb_sum_f64": [_vp, _ll, _vp, _vp, _vp],
     "smcb_scale_rows": [_vp, _ll, _i, _vp, _i, _vp, _vp],
+    "smcb_scale_rows_accepted": [_vp, _vp, _vp, _ll, _i, _vp, _vp, _vp],
     "smcb_fast_exp": [_vp, _ll, _vp, _vp],
     "smcb_fast_log": [_vp, _ll, _vp, _vp],
     "smcb_probe_fp64": [_i, _i, _i, _vp, _vp],

@@ -180,6 +180,7 @@ class NUTSProposal:
         if self.accept_reject:
             carry, want_grad = None, False
         scale = getattr(self.target, "_scale_dev", None)
+        x_in = x
         if scale is not None:   # diagonal metric: the kernel works on z = x / scale (gradients there are z-space: no carry-over)
             carry, want_grad = None, False
             z = dev.empty(N, D)
@@ -197,7 +198,10 @@ class NUTSProposal:
         if self.record_events:
             e1.record()
             self.events.append((e0, e1))
-        if scale is not None:   # back to x-space, in place
+        if scale is not None and self.accept_reject:   # back to x-space, in place; a rejected particle keeps its x row
+            _cabi.call("smcb_scale_rows_accepted", dev.ptr(o["x_new"]), dev.ptr(o["accepted"]), dev.ptr(x_in), N, D,
+                       dev.ptr(scale), dev.ptr(o["x_new"]), dev.stream_ptr())
+        elif scale is not None:                        # back to x-space, in place
             _cabi.call("smcb_scale_rows", dev.ptr(o["x_new"]), N, D, dev.ptr(scale), 0, dev.ptr(o["x_new"]), dev.stream_ptr())
         self.last = o
         return o

@@ -38,6 +38,18 @@ class DualAveragingStepSize:
         self.step_size = math.exp(log_eps)
         return self.step_size
 
+    def rescale(self, factor):
+        """The metric changed: a step of eps in the old z-units is one of eps * factor in the new ones.  The averaging
+        state moves with it (centre, current and averaged log step), and what has been learned about the acceptance
+        (h_bar, t) is kept.  Restarting instead would set mu = log(10 eps) again, and the first update after a restart
+        multiplies the step by 2.3 even at acceptance 0: with the metric changing every iteration, the step grew
+        geometrically while every tree diverged."""
+        d = math.log(float(factor))
+        self.mu += d
+        self.log_eps_bar += d if self.t else 0.0
+        self.step_size *= float(factor)
+        return self.step_size
+
     def averaged(self):
         """The step size to freeze once adaptation ends (the initial one if there was no observation)."""
         return math.exp(self.log_eps_bar) if self.t else self.step_size

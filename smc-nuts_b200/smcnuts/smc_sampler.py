@@ -180,11 +180,9 @@ class SMCSampler:
             eps = self.step_size_adapter.update(self.accept_stat[k - 1])
             if k <= self.metric_iters:
                 self._adapt_metric()
-                # the step size that suited the old metric is rescaled by the geometric mean of the change and the dual
-                # averaging starts over from there
-                self.step_size_adapter = DualAveragingStepSize(eps * self._metric_rescale,
-                                                               self.step_size_adapter.target_accept)
-                eps = self.step_size_adapter.step_size
+                # the step size that suited the old metric is rescaled by the geometric mean of the change; the dual
+                # averaging carries on in the new units (a restart per iteration grows the step whatever the acceptance)
+                eps = self.step_size_adapter.rescale(self._metric_rescale)
             if k == self.adapt_iters:
                 eps = self.step_size_adapter.averaged()
                 self.forward_kernel.want_accept_stat = False

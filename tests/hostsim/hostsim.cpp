@@ -41,17 +41,23 @@ extern "C" int hostsim_nuts(int kind, const double* data, int n_data, int dim, i
                             unsigned long long seed, unsigned iteration, unsigned long long particle0, double* x_new,
                             double* r_new, double* A_old, double* B_old, double* A_new, double* B_new, double* ke_old,
                             double* ke_new, int* n_leapfrog, int* accepted, int* depth, const double* A_in,
-                            const double* B_in, const double* g_in, double* g_new, int lanes) {
+                            const double* B_in, const double* g_in, double* g_new, int lanes, const double* scale) {
     NutsArgs a;
     std::memset(&a, 0, sizeof a);
-    a.model = ModelDesc{kind, dim, n_data, T, q, data};
+    a.model = ModelDesc{kind, dim, n_data, T, q, data, scale};
     a.x = x; a.r = r; a.N = N; a.eps = eps; a.phi = phi; a.max_depth = max_depth; a.accrej = accrej;
     a.seed = seed; a.iteration = iteration; a.particle0 = particle0;
     a.x_new = x_new; a.r_new = r_new; a.A_old = A_old; a.B_old = B_old; a.A_new = A_new; a.B_new = B_new;
     a.ke_old = ke_old; a.ke_new = ke_new; a.n_leapfrog = n_leapfrog; a.accepted = accepted; a.depth = depth;
     a.A_in = A_in; a.B_in = B_in; a.g_in = g_in; a.g_new = g_new;
-    if (kind == kArma) run<ArmaModel>(a, lanes);
-    else if (kind == kPRMwCD) run<PrmModel>(a, lanes);
-    else run<GaussModel>(a, lanes);
+    if (scale) {   // diagonal metric: x, x_new are z = x / scale (the caller converts, as proposal/nuts.py does)
+        if (kind == kArma) run<ScaledModel<ArmaModel>>(a, lanes);
+        else if (kind == kPRMwCD) run<ScaledModel<PrmModel>>(a, lanes);
+        else run<ScaledModel<GaussModel>>(a, lanes);
+    } else {
+        if (kind == kArma) run<ArmaModel>(a, lanes);
+        else if (kind == kPRMwCD) run<PrmModel>(a, lanes);
+        else run<GaussModel>(a, lanes);
+    }
     return 0;
 }

@@ -60,10 +60,30 @@ def pack_model(name, np_target):
     return 2, np.ascontiguousarray(np_target.P.ravel()), np_target.dim, 0, 0.0
 
 
-def nuts(name, np_target, x, r, eps, phi, max_depth=10, accrej=False, seed=0, iteration=0, particle0=0, lanes=32,
-         carry=None, want_grad=False, devmath=False):
-    kind, data, dim, T, q = pack_model(name, np_target)
+def _to_z(x, scale):
+    """Diagonal metric: the lanes run on z = x / scale (proposal/nuts.py converts with smcb_scale_rows)."""
     x = np.ascontiguousarray(x, dtype=np.float64)
+    if scale is None:
+        return x, None
+    scale = np.ascontiguousarray(scale, dtype=np.float64)
+    return np.ascontiguousarray(x / scale), scale
+
+
+def _to_x(o, x, scale):
+    """Back to x-space as proposal/nuts.py does: x_new = z_new * scale, except that a particle the MH epilogue rejected
+    keeps its x row (smcb_scale_rows_accepted)."""
+    if scale is not None:
+        o["x_new"] = np.where(o["accepted"][:, None] != 0, o["x_new"] * scale, x)
+    return o
+
+
+def nuts(name, np_target, x, r, eps, phi, max_depth=10, accrej=False, seed=0, iteration=0, particle0=0, lanes=32,
+         carry=None, want_grad=False, devmath=False, scale=None):
+    """One NUTS transition per particle on the one-lane kernels.  scale: diagonal metric (ScaledModel); x and x_new are
+    then x-space rows, converted as proposal/nuts.py converts them."""
+    kind, data, dim, T, q = pack_model(name, np_target)
+    x_in = np.ascontiguousarray(x, dtype=np.float64)
+    x, scale = _to_z(x_in, scale)
     r = np.ascontiguousarray(r, dtype=np.float64)
     N = len(x)
     o = dict(x_new=np.empty_like(x), r_new=np.empty_like(r), A_old=np.empty(N), B_old=np.empty(N), A_new=np.empty(N),
@@ -80,31 +100,44 @@ def nuts(name, np_target, x, r, eps, phi, max_depth=10, accrej=False, seed=0, it
                        ctypes.c_uint(iteration), ctypes.c_ulonglong(particle0), P(o["x_new"]), P(o["r_new"]),
                        P(o["A_old"]), P(o["B_old"]), P(o["A_new"]), P(o["B_new"]), P(o["ke_old"]), P(o["ke_new"]),
                        I(o["n_leapfrog"]), I(o["accepted"]), I(o["depth"]), P(cA), P(cB), P(cg), P(o.get("g_new")),
-                       ctypes.c_int(lanes))
-    return o
+                       ctypes.c_int(lanes), P(scale))
+    return _to_x(o, x_in, scale)
 
 
-def nuts_simt(name, np_target, x, r, eps, phi, max_depth=10, accrej=False, seed=0, iteration=0, particle0=0):
+def nuts_simt(name, np_target, x, r, eps, phi, max_depth=10, accrej=False, seed=0, iteration=0, particle0=0, scale=None):
     """One NUTS transition per particle on the EMULATED 4-lanes-per-particle kernels (PRMwCD: PrmModelG<13>; gauss:
-    GaussModelG<ceil(D/8)>), one persistent warp pulling particles from the work queue."""
+    GaussModelG<ceil(D/8)>), one persistent warp pulling particles from the work queue.  scale: as in nuts()."""
     kind, data, dim, T, q = pack_model(name, np_target)
     assert kind in (1, 2)
-    x = np.ascontiguousarray(x, dtype=np.float64)
+    x_in = np.ascontiguousarray(x, dtype=np.float64)
+    x, scale = _to_z(x_in, scale)
     r = np.ascontiguousarray(r, dtype=np.float64)
     N = len(x)
     o = dict(x_new=np.empty_like(x), r_new=np.empty_like(r), A_old=np.empty(N), B_old=np.empty(N), A_new=np.empty(N),
              B_new=np.empty(N), ke_old=np.empty(N), ke_new=np.empty(N), n_leapfrog=np.empty(N, dtype=np.int32),
              accepted=np.empty(N, dtype=np.int32), depth=np.empty(N, dtype=np.int32))
-    P = lambda a: a.ctypes.data_as(_dp)  # noqa: E731
+    P = lambda a: a.ctypes.data_as(_dp) if a is not None else None  # noqa: E731
     I = lambda a: a.ctypes.data_as(_ip)  # noqa: E731
     rc = lib_simt().hostsim_nuts_simt(
         ctypes.c_int(kind), P(data), ctypes.c_int(data.size), ctypes.c_int(dim), ctypes.c_int(T), ctypes.c_double(q), P(x),
         P(r), ctypes.c_longlong(N), ctypes.c_double(eps), ctypes.c_double(phi), ctypes.c_int(max_depth),
         ctypes.c_int(int(accrej)), ctypes.c_ulonglong(seed), ctypes.c_uint(iteration), ctypes.c_ulonglong(particle0),
         P(o["x_new"]), P(o["r_new"]), P(o["A_old"]), P(o["B_old"]), P(o["A_new"]), P(o["B_new"]), P(o["ke_old"]),
-        P(o["ke_new"]), I(o["n_leapfrog"]), I(o["accepted"]), I(o["depth"]))
+        P(o["ke_new"]), I(o["n_leapfrog"]), I(o["accepted"]), I(o["depth"]), P(scale))
     assert rc == 0
-    return o
+    return _to_x(o, x_in, scale)
+
+
+def scaled_probe(group, nloc, dim, scale, z):
+    """ScaledModel<probe>::eval on one emulated warp: z[32, nloc] slot values -> g[32, nloc] = s * (s * z) per slot, where
+    the probe model returns the x it sees as its gradient (hostsim_simt.cpp)."""
+    scale = np.ascontiguousarray(scale, dtype=np.float64)
+    z = np.ascontiguousarray(z, dtype=np.float64).reshape(32, nloc)
+    g = np.empty_like(z)
+    rc = lib_simt().hostsim_scaled_probe(ctypes.c_int(group), ctypes.c_int(nloc), ctypes.c_int(dim),
+                                         scale.ctypes.data_as(_dp), z.ctypes.data_as(_dp), g.ctypes.data_as(_dp))
+    assert rc == 0
+    return g
 
 
 _LIB_BISECT = None
